@@ -5,6 +5,7 @@ bench.py -- reads/sec of the counting hot path on B200 (BASELINE.json metric), O
     python bench.py [--gpus N] [--steps K] [--warmup W]            # all three workloads, see below
     python bench.py --workload bulk_pe|bulk_se|sc ...               # one workload as the headline
     python bench.py --impl reference ...                            # the unmodified reference on the host cores
+    python bench.py --dump-outputs DIR ...                          # also save the last timed step's results
 
 The headline of the line is BASELINE.json configs[3] (synthetic 500 M-record paired-end bulk on an hg38-like
 genes_tes index, SURVEY.md 8d): a "step" is one pass of filter -> overlap -> tally (+ cross-GPU merge) over the
@@ -34,6 +35,9 @@ BYTES_PER_RECORD = {"bulk_pe": 12, "bulk_se": 12, "sc": 24}        # SURVEY.md 8
 INDEX_BYTES_PER_FEATURE = 16
 CONFIG_RECORDS = {"bulk_pe": 500_000_000, "bulk_se": 500_000_000, "sc": 1_000_000_000}
 SC_RECORDS_MULTI = 250_000_000                                      # per GPU at N > 1
+DUMP_BYTES = 64_000_000                                             # --dump-outputs: 64 MB for all arrays together
+DUMP_TRIPLES = 2_000_000                                            # single-cell triples kept by the sample
+DUMP_SEED = 20261018
 
 
 def parse_args():
@@ -57,7 +61,15 @@ def parse_args():
     ap.add_argument("--file-records", type=int, default=8_000_000,
                     help="records of the synthetic BAM file of the from_file leg (0 = skip)")
     ap.add_argument("--opt", action="append", default=[], help="engine tuning knob key=value (tec_set_option)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what each timed leg returned in its last step to DIR/<leg>_<name>.npy (float64, "
+                         "at most 64 MB in all; the single-cell triples are a fixed, seeded sample)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs saves the results of --impl ours")
+    return args
 
 
 def load_peaks():
@@ -90,6 +102,33 @@ def workload_config(args, wl, n_rec_per_gpu, world):
             "sharding": "genomic coordinate range per GPU, index replicated" if world > 1 else "single GPU",
             "index_scale": args.index_scale, "l2_policy": "inputs >> L2 (no flush needed)",
             "bytes_per_record": BYTES_PER_RECORD[wl]}
+
+
+# ------------------------------------------------------------------------------ --dump-outputs
+def sample_triples(ensg, cell, count, k, seed=DUMP_SEED):
+    """The k triples whose (ensg, cell) key has the lowest seeded splitmix64 hash, in ascending key order.  The hash is
+    a bijection of the key, so which triples are kept depends on the set of triples alone, not on their order."""
+    key = ensg.astype(np.uint64) << np.uint64(32) | cell.astype(np.uint64)
+    keep = np.arange(len(key))
+    if len(key) > k:
+        z = key ^ np.uint64(seed)
+        z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+        z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+        z ^= z >> np.uint64(31)
+        keep = np.argpartition(z, k - 1)[:k] if k > 0 else keep[:0]
+    keep = keep[np.argsort(key[keep], kind="stable")]
+    return ensg[keep], cell[keep], count[keep]
+
+
+def write_outputs(path, arrays):
+    """Every array as path/<name>.npy; refuses to write more than DUMP_BYTES."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes of results exceed the limit of %d" % (total, DUMP_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    return {"dir": os.path.abspath(path), "arrays": len(arrays), "bytes": int(total)}
 
 
 # ------------------------------------------------------------------------------ clocks sampler
@@ -224,16 +263,16 @@ def run_reference(args):
 
     head = bulk(wl == "bulk_pe", K, W, n) if wl in ("bulk_pe", "bulk_se") else None
     if args.workload == "all":
-        legs["bulk_se"] = bulk(False, 2, 1, n)
+        legs["bulk_se"] = bulk(False, K, W, n)
     if args.workload in ("all", "sc"):
         n_sc = max(1000, n // 3)
         r = synth.synth_sc_reads(synth.SEED, idx, n_sc, n_whitelist=100_000)
         arrays = [r[k] for k in ("start", "end", "chrom", "mapq", "flag", "cell", "umi")]
         ts = []
-        for _ in range(2 if args.workload == "all" else W + K):
+        for _ in range(W + K):
             dt, res, mte = reference_time_sc(R, arrays, 100_000, True, 10_000)
             ts.append(dt)
-        ts = ts[1:] if len(ts) > 1 else ts
+        ts = ts[W:]
         sc = {"value": n_sc / float(np.mean(ts)), "unit": "records/s", "ms_per_step": 1e3 * float(np.mean(ts)), "steps": len(ts),
               "records_per_step": n_sc, "what": "measureTE.sc_parse_bamse(strand=True, maxcells=10000), 100 k-barcode whitelist; "
               "load_genome bound to a no-op on the instance (index object already in place)"}
@@ -346,6 +385,23 @@ class Ctx:
         self.ext = torch.cuda.ExternalStream(self.eng.stream, device=self.dev)
         self.peak, self.peak_src = load_peaks()
         self._ref = None
+        self.outputs = {}
+
+    def keep_outputs(self, leg, **arrays):
+        """--dump-outputs: results of a leg's last timed step, as float64 (exact for these integers, all below 2**53)."""
+        if self.args.dump_outputs and self.rank == 0:
+            for name, a in arrays.items():
+                self.outputs[leg + "_" + name] = np.asarray(a, dtype=np.float64).reshape(-1)
+
+    def keep_sc_outputs(self, ensg, cell, count, hit_cell, hit_count, stats, selected, n_triples):
+        """The single-cell results; the triples as a sample of at most DUMP_TRIPLES that fits what is left of
+        DUMP_BYTES after every other array (3 float64 columns, 24 bytes per triple)."""
+        if not (self.args.dump_outputs and self.rank == 0):
+            return
+        self.keep_outputs("sc", stats=stats, hit_cell=hit_cell, hit_count=hit_count, selected=selected, n_triples=[n_triples])
+        used = sum(a.nbytes for a in self.outputs.values())
+        k = max(0, min(DUMP_TRIPLES, (DUMP_BYTES - used) // 24))
+        self.keep_outputs("sc", **dict(zip(("ensg", "cell", "count"), sample_triples(ensg, cell, count, k))))
 
     def barrier(self):
         if self.world > 1:
@@ -424,6 +480,7 @@ def bulk_leg(C, wl, headline):
     ms_step = C.max_over_ranks(e0.elapsed_time(e1)) / K
     value = n_rec * world / (ms_step / 1e3)
     counts, st = eng.bulk_finish()
+    C.keep_outputs(wl, counts=counts, stats=st)
 
     # ---- end to end through the host-buffer ABI (pinned host arrays, H2D + D2H in the timed region)
     parity_full = None
@@ -444,7 +501,7 @@ def bulk_leg(C, wl, headline):
         for _ in range(2):
             c2, s2 = e2e_step()
         C.barrier()
-        Ke = K if headline else min(K, 3)
+        Ke = K
         ta = time.perf_counter()
         for _ in range(Ke):
             c2, s2 = e2e_step()
@@ -610,7 +667,7 @@ def sc_leg(C, headline):
         return nt, nh, sel
 
     W = max(3, args.warmup) if headline else 3
-    K = args.steps if headline else min(args.steps, 5)
+    K = args.steps
     for _ in range(W):
         step()
     C.barrier()
@@ -636,6 +693,7 @@ def sc_leg(C, headline):
         ms_step = C.max_over_ranks(max(ms_step, (t1 - t0) * 1e3 / K))
     value = n_rec * world / (ms_step / 1e3)
     ensg, cell, count, hcell, hcount, st = eng.sc_fetch(nt, nh)
+    C.keep_sc_outputs(ensg, cell, count, hcell, hcount, st, sel, nt)
     # dense matrix rows of sc_save_result formatted on the device (te_count.py:744-754): size and rate
     matrix_text = None
     if world == 1 and len(sel) and headline:
@@ -671,7 +729,7 @@ def sc_leg(C, headline):
             return out, eng.sc_select(maxcells, b)
 
         e2e_step()
-        Ke = min(K, 3)
+        Ke = K
         ta = time.perf_counter()
         for _ in range(Ke):
             out2, sel2 = e2e_step()
@@ -815,6 +873,8 @@ def run_ours(args):
             line[k] = head[k]
     line.update(legs)
     line["bench_seconds"] = time.time() - t_start
+    if args.dump_outputs and C.rank == 0:
+        line["dump_outputs"] = write_outputs(args.dump_outputs, C.outputs)
     if C.rank == 0:
         print(json.dumps(line))
     C.eng.close()
