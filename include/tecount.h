@@ -279,9 +279,8 @@ const char *tec_bam_reference_name(const tec_bam *b, int i);
 int tec_bam_set_chrom_map(tec_bam *b, const uint16_t *bulk_ids, const uint16_t *sc_ids, int32_t n, int32_t n_index);
 int tec_bam_set_whitelist(tec_bam *b, const char *barcodes, const int64_t *offsets, int32_t n);
 int tec_bam_count(tec_bam *b, int mode, int qual, int64_t *n_records);
-/* One BYTE RANGE of the file, for several ranks that split one BAM (single end and single cell; pairs are formed by
- * the global record parity and stay with one decoder).  Counts the records that START in the BGZF blocks whose first
- * byte lies in [byte_lo, byte_hi) into the running count.  out[TEC_BAM_RANGE_WORDS] = {records counted, start_block,
+/* One BYTE RANGE of the file, for several ranks that split one BAM.  Counts the records that START in the BGZF blocks
+ * whose first byte lies in [byte_lo, byte_hi) into the running count.  out[TEC_BAM_RANGE_WORDS] = {records counted, start_block,
  * start_off, exit_block, exit_off, file size}: where this range's first record starts and where the chain stands
  * behind its last record, each as {file offset of the BGZF block, offset in its inflated data}.  start_block -1: the
  * range began at the BAM header (byte_lo == 0, exact); -2: no record starts in the range.  The first record of any other
@@ -289,6 +288,26 @@ int tec_bam_count(tec_bam *b, int mode, int qual, int64_t *n_records);
  * rank and exit(last) == {file size, 0}; if that fails, decode the file in one piece (te_count.py does both). */
 #define TEC_BAM_RANGE_WORDS 6
 int tec_bam_count_range(tec_bam *b, int mode, int qual, int64_t byte_lo, int64_t byte_hi, int64_t *out);
+/* Paired end (mode 1) over byte ranges.  The reference pairs records by their GLOBAL index (record 2i is read1,
+ * 2i+1 read2, a trailing odd record is dropped), which a range does not know until the ranges in front of it are
+ * counted.  So tec_bam_count_range(b, 1, ...) counts every adjacent pair (j, j+1) of the range (j = range-local index)
+ * into one of two counter banks, bank j & 1, both starting from the running count; out[0] is still the number of
+ * records.  Once the caller knows the range's global offset o (the sum of the record counts of the ranges in front):
+ *   tec_bulk_keep_bank(ctx, o & 1)   makes that bank the running count and drops the other.  Until it is called,
+ *                                    tec_bulk_push*, tec_bulk_allreduce, tec_bulk_finish, tec_bam_count and
+ *                                    tec_bam_count_range return TEC_ERR_STATE; tec_bulk_begin clears that state.
+ *   if o is odd and the range has records, its first record is read2 of a pair whose read1 is the last record of the
+ *   nearest range in front that has records: tec_bam_pair_columns parses the two, tec_bulk_push counts them.
+ * tec_bam_range_record: raw bytes (block_size word included) of the first (which = 0) or last (which = 1) record of
+ * the last paired-end tec_bam_count_range on b; *len = their number (0: no record, or another mode).  buf = NULL only
+ * asks for the length; otherwise cap must be at least *len.
+ * tec_bam_pair_columns: read1 = rec1[0, n1), read2 = rec2[0, n2), each one raw record of this file, parsed on the host
+ * with b's chromosome map into rows 0 and 1 (the record layout above), with the same rules and the same status as the
+ * device parse (TEC_ERR_FORMAT for a malformed record, TEC_ERR_ARG when a buffer is not one whole record). */
+int tec_bulk_keep_bank(tec_ctx *ctx, int bank);
+int tec_bam_range_record(const tec_bam *b, int which, void *buf, int64_t cap, int64_t *len);
+int tec_bam_pair_columns(tec_bam *b, const void *rec1, int64_t n1, const void *rec2, int64_t n2, int qual,
+                         int32_t *start, int32_t *end, uint16_t *chrom, uint8_t *mapq, uint8_t *flag);
 /* what = 0 blocks inflated by zlib on the host, 1..4 microseconds in load / inflate / chain / parse */
 int64_t tec_bam_info(const tec_bam *b, int what);
 

@@ -63,6 +63,9 @@ SIGNATURES = {
     "tec_bam_set_whitelist": (ctypes.c_int, [_vp, ctypes.c_char_p, _vp, ctypes.c_int32]),
     "tec_bam_count": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, _c_i64p]),
     "tec_bam_count_range": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int64, ctypes.c_int64, _c_i64p]),
+    "tec_bam_range_record": (ctypes.c_int, [_vp, ctypes.c_int, _vp, ctypes.c_int64, _c_i64p]),
+    "tec_bam_pair_columns": (ctypes.c_int, [_vp, _vp, ctypes.c_int64, _vp, ctypes.c_int64, ctypes.c_int, _vp, _vp, _vp, _vp, _vp]),
+    "tec_bulk_keep_bank": (ctypes.c_int, [_vp, ctypes.c_int]),
     "tec_bam_info": (ctypes.c_int64, [_vp, ctypes.c_int]),
     "tec_sc_matrix_text": (ctypes.c_int, [_vp, ctypes.c_int64, _c_u32p, ctypes.c_char_p, _c_i64p, _c_i64p]),
     "tec_sc_matrix_read": (ctypes.c_int, [_vp, ctypes.c_int64, ctypes.c_int64, _vp]),
@@ -182,12 +185,35 @@ class DeviceBam:
 
     def count_range(self, mode, qual, byte_lo, byte_hi):
         """The records that start in the BGZF blocks of [byte_lo, byte_hi) (include/tecount.h: tec_bam_count_range).
-        Returns {n, start, exit, size}: start / exit are (block file offset, offset in the inflated block)."""
+        Returns {n, start, exit, size}: start / exit are (block file offset, offset in the inflated block).  Paired end
+        (mode 1) adds first / last: the raw bytes of the range's first and last record (b"" without records); the
+        engine then waits for Engine.bulk_keep_bank."""
         out = (ctypes.c_int64 * 6)()
         rc = self._lib.tec_bam_count_range(self._h, int(mode), int(qual), int(byte_lo), int(byte_hi), out)
-        if rc == 0:
-            return {"n": out[0], "start": (out[1], out[2]), "exit": (out[3], out[4]), "size": out[5]}
-        self._raise(rc, mode)
+        if rc != 0:
+            self._raise(rc, mode)
+        info = {"n": out[0], "start": (out[1], out[2]), "exit": (out[3], out[4]), "size": out[5]}
+        if int(mode) == 1:
+            info["first"], info["last"] = self._range_record(0), self._range_record(1)
+        return info
+
+    def _range_record(self, which):
+        n = ctypes.c_int64(0)
+        self._eng._check(self._lib.tec_bam_range_record(self._h, which, None, 0, ctypes.byref(n)))
+        buf = ctypes.create_string_buffer(max(1, n.value))
+        self._eng._check(self._lib.tec_bam_range_record(self._h, which, buf, n.value, ctypes.byref(n)))
+        return buf.raw[:n.value]
+
+    def pair_columns(self, rec1, rec2, qual):
+        """read1 = rec1, read2 = rec2 (raw records of this file, e.g. count_range's last / first) parsed on the host with
+        this file's chromosome map: {start, end, chrom, mapq, flag}, two rows each, the layout bulk_push takes."""
+        cols = {"start": np.zeros(2, np.int32), "end": np.zeros(2, np.int32), "chrom": np.zeros(2, np.uint16),
+                "mapq": np.zeros(2, np.uint8), "flag": np.zeros(2, np.uint8)}
+        rc = self._lib.tec_bam_pair_columns(self._h, rec1, len(rec1), rec2, len(rec2), int(qual),
+                                            *[cols[k].ctypes.data for k in ("start", "end", "chrom", "mapq", "flag")])
+        if rc != 0:
+            self._raise(rc, 1)
+        return cols
 
     def _raise(self, rc, mode):
         msg = (self._lib.tec_last_error(self._eng._h) or b"").decode()
@@ -346,6 +372,10 @@ class Engine:
         self._check(self._lib.tec_bulk_finish(self._h, ctypes.cast(counts.ctypes.data, _c_i64p),
                                               ctypes.cast(stats.ctypes.data, _c_i64p)))
         return counts, stats
+
+    def bulk_keep_bank(self, bank):
+        """after a paired-end count_range: keep counter bank `bank` (the parity of the range's global record offset)"""
+        self._check(self._lib.tec_bulk_keep_bank(self._h, int(bank)))
 
     def bulk_counts_dev(self):
         return self._lib.tec_bulk_counts_dev(self._h)

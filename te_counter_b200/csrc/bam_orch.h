@@ -233,7 +233,36 @@ struct Reader {
         }
         return OK;
     }
+
+    // the parse context over the host copies of the maps
+    bgzfdev::ParseCtx host_parse_ctx(int qual) const {
+        bgzfdev::ParseCtx pc;
+        pc.bulk_ids = bulk_ids.data(); pc.sc_ids = sc_ids.data(); pc.n_ref = (int32_t)refs.size(); pc.n_index = n_index; pc.qual = qual;
+        pc.wl.slot = wl_slot.data(); pc.wl.off = wl_off.data(); pc.wl.bytes = (const uint8_t*)wl_bytes.data();
+        pc.wl.mask = wl_slot.empty() ? 0 : wl_slot.size() - 1;
+        return pc;
+    }
 };
+
+// One paired-end pair parsed on the host from two raw records (block_size word included), with the file's chromosome
+// map: the pair across the border of two byte ranges (decode_range).  Same routine as the device pass, rows 0 and 1.
+inline int parse_pair(Reader& r, const uint8_t* rec1, int64_t n1, const uint8_t* rec2, int64_t n2, int qual,
+                      int32_t* start, int32_t* end, uint16_t* chrom, uint8_t* mapq, uint8_t* flag) {
+    if (!r.have_map) return r.fail(E_ARG, "the chromosome map has not been set");
+    auto whole = [](const uint8_t* p, int64_t n) {
+        return n >= 36 && n <= 4 + (int64_t)bgzfdev::MAX_BLOCK_SIZE && (int64_t)bgzfdev::ld32(p) + 4 == n;
+    };
+    if (!whole(rec1, n1) || !whole(rec2, n2)) return r.fail(E_ARG, "a mate is not one complete alignment record");
+    std::vector<uint8_t> w((size_t)(n1 + n2));
+    memcpy(w.data(), rec1, (size_t)n1);
+    memcpy(w.data() + n1, rec2, (size_t)n2);
+    const int64_t off[2] = {0, n1};
+    const bgzfdev::ParseCtx pc = r.host_parse_ctx(qual);
+    const bgzfdev::Columns set{start, end, chrom, mapq, flag, nullptr, nullptr};
+    const int e = bgzfdev::parse_adjacent_pair(w.data(), off, 0, 0, pc, &set);
+    if (e) return r.fail(E_RECORD - e, "the pair across the range border");
+    return OK;
+}
 
 /*
  * Backend concept:
@@ -246,6 +275,11 @@ struct Reader {
  *   int  parse(const BlockDesc*, int n_blocks, const BlockChain* used, const int64_t* base, int64_t n_records, int64_t w_end,
  *              int mode, int qual, const Reader&, int* err, int64_t* err_rec)                 parse_record per record into the columns
  *   int  deliver(int64_t n_records, int mode)                          hand the columns on (tec_*_push_dev / copy out)
+ * and for paired-end byte ranges (decode_range with MODE_PE):
+ *   int  parse_pairs(const BlockChain*, const int64_t* base, int nb, int64_t n_records, int64_t g0, int qual, const Reader&,
+ *                    int* err, int64_t* err_rec)                       parse_adjacent_pair per adjacent pair into the two column sets
+ *   int  deliver_pairs(int64_t pairs0, int64_t pairs1)                 hand column set b on to counter bank b
+ *   int  fetch(int64_t at, uint8_t* dst, size_t n)                     window bytes to the host
  */
 template <class Backend>
 int decode_all(Reader& r, Backend& be, int mode, int qual, int window_blocks, int64_t* n_records_out) {
@@ -391,14 +425,29 @@ int decode_all(Reader& r, Backend& be, int mode, int qual, int window_blocks, in
 // The caller compares every rank's exit with the next rank's start (both as {file offset of the block, offset inside
 // its inflated data}): by induction from rank 0, whose start is exact, equality everywhere means every rank decoded
 // exactly its share of the true record chain; any difference means a wrong guess and the caller must decode the file
-// in one piece instead.  Single-end and single-cell modes only (pairs are formed by global record parity).
+// in one piece instead.
+// Paired end: pairs are formed by the GLOBAL record parity, which a range does not know until the ranks in front of it
+// have counted their records.  So every adjacent pair (j, j + 1) of the range (range-local indices) is parsed, into
+// column set j & 1 (parse_pairs / deliver_pairs: two counter banks); the caller keeps the set of the range's global
+// offset once it is known, and parses the pair across the border from the raw first / last records kept here.  The last
+// complete record of a window is carried into the next one, so the pair across two windows is formed exactly once.
 constexpr int RANGE_TAIL_BLOCKS = 16;               // blocks behind the range that are inflated for its last record:
 constexpr size_t RANGE_TAIL_BYTES = size_t(1) << 20;   // at least 16 of them and at least 1 MiB of inflated data
 struct RangeResult {
     int64_t n_records = 0;
     int64_t start_block = -1, start_off = 0;      // -1: the range starts at the BAM header (exact); -2: no record starts in the range
     int64_t exit_block = -2, exit_off = 0;        // where the next record starts; block == file size: end of file
+    std::vector<uint8_t> first_rec, last_rec;     // paired end: raw bytes (block_size word included) of the first / last record
 };
+
+// raw bytes of the record at window offset p (block_size word included)
+template <class Backend>
+int fetch_record(Backend& be, int64_t p, std::vector<uint8_t>& out) {
+    uint8_t w[4];
+    if (be.fetch(p, w, 4)) return 1;
+    out.resize(4 + (size_t)bgzfdev::ld32(w));
+    return be.fetch(p, out.data(), out.size());
+}
 
 inline bool bgzf_chain_ok(const MappedFile& f, size_t p, int n) {
     for (int i = 0; i < n && p < f.size; i++) {
@@ -413,10 +462,11 @@ inline bool bgzf_chain_ok(const MappedFile& f, size_t p, int n) {
 template <class Backend>
 int decode_range(Reader& r, Backend& be, int mode, int qual, int window_blocks, uint64_t lo, uint64_t hi, RangeResult* res) {
     if (!r.have_map) return r.fail(E_ARG, "the chromosome map has not been set");
-    if (mode == bgzfdev::MODE_PE) return r.fail(E_ARG, "byte ranges are for single-end and single-cell decoding (pairs follow the global record parity)");
     if (!res || lo > hi) return r.fail(E_ARG, "bad byte range");
     if (window_blocks < 1) window_blocks = 1;
     *res = RangeResult();
+    const bool paired = mode == bgzfdev::MODE_PE;
+    int64_t carried = 0;                        // paired: the window begins with a record an earlier window counted (0 or 1)
     const size_t fsize = r.file.size;
     const size_t hi_eff = (size_t)std::min<uint64_t>(hi, fsize);
     const bool from_header = lo == 0;           // rank 0: the chain starts behind the BAM header, exactly
@@ -522,6 +572,7 @@ int decode_range(Reader& r, Backend& be, int mode, int qual, int window_blocks, 
         if (be.chain(blocks.data(), nc, w_end, (int32_t)r.refs.size(), chain.data())) return r.fail(E_BACKEND, "backend: chain pass failed");
         int64_t expect = 0, n_rec = 0;
         bool stopped = false;
+        int first_used = -1, last_used = -1;
         for (int b = 0; b < nc; b++) {
             const int64_t lo_b = (int64_t)blocks[(size_t)b].out_off, hi_b = lo_b + blocks[(size_t)b].out_len;
             BlockChain& c = chain[(size_t)b];
@@ -543,6 +594,7 @@ int decode_range(Reader& r, Backend& be, int mode, int qual, int window_blocks, 
             }
             if (c.bad) return r.fail(E_FORMAT, "alignment record with impossible block_size");
             n_rec += c.count;
+            if (c.count) { if (first_used < 0) first_used = b; last_used = b; }
             expect = c.exit;
             if (c.exit < hi_b) stopped = true;
         }
@@ -550,7 +602,31 @@ int decode_range(Reader& r, Backend& be, int mode, int qual, int window_blocks, 
         base.assign((size_t)nc, 0);
         int64_t acc = 0;
         for (int b = 0; b < nc; b++) { base[(size_t)b] = acc; acc += chain[(size_t)b].count; }
-        if (n_rec) {
+        if (paired && n_rec) {
+            // n_rec complete records, the carried one included: n_rec - 1 adjacent pairs, the first record at range index g0
+            const int64_t g0 = total_records - carried;
+            if (res->first_rec.empty() && fetch_record(be, chain[(size_t)first_used].start, res->first_rec))
+                return r.fail(E_BACKEND, "backend: copy failed");
+            if (fetch_record(be, chain[(size_t)last_used].last, res->last_rec)) return r.fail(E_BACKEND, "backend: copy failed");
+            if (n_rec > 1) {
+                int err = 0;
+                int64_t err_rec = -1;
+                if (be.parse_pairs(chain.data(), base.data(), nc, n_rec, g0, qual, r, &err, &err_rec))
+                    return r.fail(E_BACKEND, "backend: parse pass failed");
+                if (err) {
+                    char buf[96];
+                    snprintf(buf, sizeof buf, "record %lld of the range", (long long)(g0 + err_rec));
+                    return r.fail(E_RECORD - err, buf);
+                }
+                if (be.deliver_pairs(bgzfdev::pairs_in_set(n_rec, g0, 0), bgzfdev::pairs_in_set(n_rec, g0, 1)))
+                    return r.fail(E_BACKEND, "backend: delivering the batch failed");
+            }
+            total_records += n_rec - carried;
+            if (!final_window) {                                 // the last record pairs with the first one of the next window
+                expect = chain[(size_t)last_used].last;
+                carried = 1;
+            }
+        } else if (n_rec) {
             int err = 0;
             int64_t err_rec = -1;
             if (be.parse(blocks.data(), nc, chain.data(), base.data(), n_rec, w_end, mode, qual, r, &err, &err_rec))

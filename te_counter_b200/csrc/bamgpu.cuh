@@ -98,6 +98,21 @@ __global__ void bam_parse_kernel(int64_t n_rec, const int64_t* __restrict__ rec_
     }
 }
 
+struct PairSets {
+    bgzfdev::Columns s[2];
+};
+
+// paired-end byte range: one thread per ADJACENT pair i (records i, i + 1 of the window), written into the column set of
+// the parity of its range-local index g0 + i (bgzfdev::parse_adjacent_pair); every record is parsed once as read1 and
+// once as read2, in the two sets
+__global__ void bam_parse_pairs_kernel(int64_t n_pairs, const int64_t* __restrict__ rec_off, const uint8_t* __restrict__ ubuf, int64_t g0,
+                                       bgzfdev::ParseCtx pc, PairSets sets, unsigned long long* __restrict__ first_err) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_pairs; i += (int64_t)gridDim.x * blockDim.x) {
+        const int e = bgzfdev::parse_adjacent_pair(ubuf, rec_off, i, g0, pc, sets.s);
+        if (e) atomicMin(first_err, ((unsigned long long)i << 8) | (unsigned long long)e);
+    }
+}
+
 struct BamGpuBackend {
     tec_ctx* ctx;
     uint8_t *d_comp = nullptr, *d_ubuf = nullptr, *d_scratch = nullptr, *d_tmp = nullptr;
@@ -117,6 +132,9 @@ struct BamGpuBackend {
     bool ctx_uploaded = false;
     bgzfdev::Columns col{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     int64_t col_cap = 0;
+    PairSets pairs{};                      // paired-end ranges: the two column sets (separate allocations: aligned for bulk2)
+    int64_t* d_pair_off = nullptr;
+    int64_t pairs_cap = 0;
     int64_t n_declined = 0;
     double ms_load = 0, ms_inflate = 0, ms_chain = 0, ms_parse = 0;
 
@@ -125,7 +143,9 @@ struct BamGpuBackend {
         cudaSetDevice(ctx->device);
         cudaStreamSynchronize(ctx->stream);
         void* blocks[] = {d_comp, d_ubuf, d_scratch, d_tmp, d_blocks, d_chain, d_base, d_status, d_crc, d_err, d_bulk_ids, d_sc_ids, d_wl_slot,
-                          d_wl_off, d_wl_bytes, d_rec_off, col.start, col.end, col.chrom, col.mapq, col.flag, col.cell, col.umi};
+                          d_wl_off, d_wl_bytes, d_rec_off, col.start, col.end, col.chrom, col.mapq, col.flag, col.cell, col.umi, d_pair_off,
+                          pairs.s[0].start, pairs.s[0].end, pairs.s[0].chrom, pairs.s[0].mapq, pairs.s[0].flag,
+                          pairs.s[1].start, pairs.s[1].end, pairs.s[1].chrom, pairs.s[1].mapq, pairs.s[1].flag};
         for (void* p : blocks) ctx->cache.put(p);            // back to the context's block cache: the next file reuses them
     }
     template <class T> cudaError_t dev_alloc(T** out, size_t bytes) {
@@ -309,9 +329,7 @@ struct BamGpuBackend {
         if (n) BAM_CK(cudaMemcpy(*dst, src, n, cudaMemcpyHostToDevice));
         return 0;
     }
-    int parse(const bamorch::BlockDesc*, int nb, const bamorch::BlockChain* ch, const int64_t* base, int64_t n, int64_t, int mode, int qual,
-              const bamorch::Reader& r, int* err, int64_t* err_rec) {
-        const double t0 = now_ms();
+    int upload_maps(const bamorch::Reader& r) {
         if (!ctx_uploaded) {
             if (up(&d_bulk_ids, r.bulk_ids.data(), r.bulk_ids.size() * 2) || up(&d_sc_ids, r.sc_ids.data(), r.sc_ids.size() * 2) ||
                 up(&d_wl_slot, r.wl_slot.data(), r.wl_slot.size() * 4) || up(&d_wl_off, r.wl_off.data(), r.wl_off.size() * 8) ||
@@ -319,6 +337,12 @@ struct BamGpuBackend {
                 return 1;
             ctx_uploaded = true;
         }
+        return 0;
+    }
+    int parse(const bamorch::BlockDesc*, int nb, const bamorch::BlockChain* ch, const int64_t* base, int64_t n, int64_t, int mode, int qual,
+              const bamorch::Reader& r, int* err, int64_t* err_rec) {
+        const double t0 = now_ms();
+        if (upload_maps(r)) return 1;
         if (n > col_cap) {
             BAM_CK(cudaStreamSynchronize(ctx->stream));
             dev_free(col.start); dev_free(col.end); dev_free(col.chrom); dev_free(col.mapq); dev_free(col.flag); dev_free(col.cell); dev_free(col.umi);
@@ -361,12 +385,60 @@ struct BamGpuBackend {
         ms_parse += now_ms() - t0;
         return 0;
     }
+    int parse_pairs(const bamorch::BlockChain* ch, const int64_t* base, int nb, int64_t n, int64_t g0, int qual, const bamorch::Reader& r,
+                    int* err, int64_t* err_rec) {
+        const double t0 = now_ms();
+        if (upload_maps(r)) return 1;
+        if (n > pairs_cap) {               // each set holds at most n rows (n - 1 pairs, every other one)
+            BAM_CK(cudaStreamSynchronize(ctx->stream));
+            for (bgzfdev::Columns& s : pairs.s) { dev_free(s.start); dev_free(s.end); dev_free(s.chrom); dev_free(s.mapq); dev_free(s.flag); }
+            dev_free(d_pair_off);
+            pairs_cap = 0;
+            const size_t cap = (size_t)n + ((size_t)n >> 3) + 1024;
+            for (bgzfdev::Columns& s : pairs.s) {
+                BAM_CK(dev_alloc(&s.start, cap * 4)); BAM_CK(dev_alloc(&s.end, cap * 4)); BAM_CK(dev_alloc(&s.chrom, cap * 2));
+                BAM_CK(dev_alloc(&s.mapq, cap)); BAM_CK(dev_alloc(&s.flag, cap));
+            }
+            BAM_CK(dev_alloc(&d_pair_off, cap * 8));
+            pairs_cap = (int64_t)cap;
+        }
+        bgzfdev::ParseCtx pc;
+        pc.bulk_ids = d_bulk_ids; pc.sc_ids = d_sc_ids; pc.n_ref = (int32_t)r.refs.size(); pc.n_index = r.n_index; pc.qual = qual;
+        pc.wl.slot = d_wl_slot; pc.wl.off = d_wl_off; pc.wl.bytes = d_wl_bytes; pc.wl.mask = r.wl_slot.empty() ? 0 : r.wl_slot.size() - 1;
+        BAM_CK(cudaMemcpyAsync(d_chain, ch, sizeof(bamorch::BlockChain) * (size_t)nb, cudaMemcpyHostToDevice, ctx->stream));
+        BAM_CK(cudaMemcpyAsync(d_base, base, 8 * (size_t)nb, cudaMemcpyHostToDevice, ctx->stream));
+        BAM_CK(cudaMemsetAsync(d_err, 0xFF, 8, ctx->stream));
+        bam_list_kernel<<<(nb + BAM_TPB - 1) / BAM_TPB, BAM_TPB, 0, ctx->stream>>>(nb, d_chain, d_base, d_ubuf, d_pair_off);
+        BAM_CK(cudaGetLastError());
+        const int64_t n_pairs = n - 1;
+        const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((n_pairs + 127) / 128, (int64_t)ctx->n_sm * 64));
+        bam_parse_pairs_kernel<<<grid, 128, 0, ctx->stream>>>(n_pairs, d_pair_off, d_ubuf, g0, pc, pairs, d_err);
+        BAM_CK(cudaGetLastError());
+        unsigned long long e = 0;
+        BAM_CK(cudaMemcpyAsync(&e, d_err, 8, cudaMemcpyDeviceToHost, ctx->stream));
+        BAM_CK(cudaStreamSynchronize(ctx->stream));
+        *err = 0;
+        if (e != ~0ull) {
+            *err = (int)(e & 0xFF);
+            *err_rec = (int64_t)(e >> 8);
+        }
+        ctx->launches += 2;
+        ms_parse += now_ms() - t0;
+        return 0;
+    }
+    int fetch(int64_t at, uint8_t* dst, size_t n) {
+        BAM_CK(cudaMemcpyAsync(dst, d_ubuf + at, n, cudaMemcpyDeviceToHost, ctx->stream));
+        BAM_CK(cudaStreamSynchronize(ctx->stream));
+        return 0;
+    }
     int deliver(int64_t n, int mode);
+    int deliver_pairs(int64_t pairs0, int64_t pairs1);
 };
 
 struct tec_bam {
     tec_ctx* ctx;
     bamorch::Reader reader;
     BamGpuBackend be;
+    std::vector<uint8_t> edge[2];          // first / last record of the last paired-end range (tec_bam_range_record)
     explicit tec_bam(tec_ctx* c) : ctx(c), be(c) {}
 };

@@ -678,4 +678,16 @@ BGZF_HD int parse_record(const uint8_t* w, int64_t p, int64_t p2, int mode, cons
     return E_NONE;
 }
 
+// Paired end over a byte range whose first record has an unknown global parity: adjacent pair i of a
+// window (records at rec_off[i] and rec_off[i + 1]; record 0 of the window has range-local index g0) is
+// read1 + read2 if g0 + i has the parity of the range's global offset.  Both candidates are kept: the pair
+// goes to column set (g0 + i) & 1 as rows 2 (i >> 1) and 2 (i >> 1) + 1, so each set holds its pairs in
+// file order.  Returns E_*.
+BGZF_HD int parse_adjacent_pair(const uint8_t* w, const int64_t* rec_off, int64_t i, int64_t g0, const ParseCtx& pc, const Columns* sets) {
+    return parse_record(w, rec_off[i], rec_off[i + 1], MODE_PE, pc, sets[(g0 + i) & 1], 2 * (i >> 1));
+}
+
+// rows of column set `bank` from the m records of a window that starts at range-local index g0 (m - 1 adjacent pairs)
+BGZF_HD int64_t pairs_in_set(int64_t m, int64_t g0, int bank) { return m > 0 ? (m - ((bank - g0) & 1)) / 2 : 0; }
+
 }  // namespace bgzfdev

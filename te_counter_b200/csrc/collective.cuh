@@ -130,6 +130,7 @@ static int comm_allreduce(tec_ctx* ctx, void* dev, int64_t count, int dtype, int
 extern "C" int tec_bulk_allreduce(tec_ctx* ctx) {
     if (!ctx) return TEC_ERR_ARG;
     if (!ctx->bulk_active) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_allreduce: tec_bulk_begin not called");
+    if (ctx->bank_pending) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_allreduce: a paired-end range count waits for tec_bulk_keep_bank");
     if (!ctx->comm) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_allreduce: tec_comm_init not called");
     TEC_CUDA(cudaSetDevice(ctx->device));
     return comm_allreduce(ctx, ctx->d_counts, (int64_t)ctx->idx.n_ensg + TEC_BULK_NSTATS, 1, 0);

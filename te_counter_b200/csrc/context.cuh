@@ -151,6 +151,8 @@ struct tec_ctx {
     bool bulk_active = false;
     int paired = 0, qual = 20;
     u64* d_counts = nullptr;              // n_ensg counters (slot order) + TEC_BULK_NSTATS statistics
+    u64* d_bank1 = nullptr;               // paired-end byte range: the counters of the pairs of odd range-local index (same layout)
+    bool bank_pending = false;            // a paired-end range count waits for tec_bulk_keep_bank
     u32* d_slow_list = nullptr;           // [0] = count, then unit indices flagged for bulk_slow_kernel
     int64_t slow_cap = 0;                 // words
     void* d_ring = nullptr;               // per-warp second deferral ring of the fast bulk kernel (QEnt)
@@ -234,6 +236,9 @@ inline void tec_ctx::free_index() {
     ix = DevIndex();
     cudaFree(d_counts);
     d_counts = nullptr;
+    cudaFree(d_bank1);
+    d_bank1 = nullptr;
+    bank_pending = false;
     cudaFree(d_slow_list);
     d_slow_list = nullptr;
     cudaFree(d_ring); cudaFree(d_ring_u);

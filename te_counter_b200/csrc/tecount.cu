@@ -333,6 +333,14 @@ extern "C" int tec_bulk_begin(tec_ctx* ctx, int paired, int qual) {
     ctx->qual = qual;
     TEC_CUDA(cudaMemsetAsync(ctx->d_counts, 0, ((size_t)ctx->idx.n_ensg + TEC_BULK_NSTATS) * 8, ctx->stream));
     ctx->bulk_active = true;
+    ctx->bank_pending = false;
+    return TEC_OK;
+}
+
+// the checks of tec_bulk_push* / tec_bulk_finish / tec_bulk_allreduce: begun, and no paired-end range waiting for its bank
+static int bulk_ready(tec_ctx* ctx, const char* what) {
+    if (!ctx->bulk_active) TEC_FAIL(TEC_ERR_STATE, std::string(what) + ": tec_bulk_begin not called");
+    if (ctx->bank_pending) TEC_FAIL(TEC_ERR_STATE, std::string(what) + ": a paired-end range count waits for tec_bulk_keep_bank");
     return TEC_OK;
 }
 
@@ -546,10 +554,8 @@ static int bulk_launch(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const 
     return TEC_OK;
 }
 
-extern "C" int tec_bulk_push_dev(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const int32_t* end,
-                                 const uint16_t* chrom, const uint8_t* mapq, const uint8_t* flag) {
-    if (!ctx) return TEC_ERR_ARG;
-    if (!ctx->bulk_active) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_push_dev: tec_bulk_begin not called");
+static int bulk_push_dev(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const int32_t* end,
+                         const uint16_t* chrom, const uint8_t* mapq, const uint8_t* flag) {
     if (n_rec < 0 || (ctx->paired && (n_rec & 1))) TEC_FAIL(TEC_ERR_ARG, "tec_bulk_push_dev: record count must be even in paired mode");
     if (n_rec == 0) return TEC_OK;
     if (!start || !end || !chrom || !mapq || !flag) TEC_FAIL(TEC_ERR_ARG, "tec_bulk_push_dev: null array");
@@ -564,12 +570,19 @@ extern "C" int tec_bulk_push_dev(tec_ctx* ctx, int64_t n_rec, const int32_t* sta
     return TEC_OK;
 }
 
+extern "C" int tec_bulk_push_dev(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const int32_t* end,
+                                 const uint16_t* chrom, const uint8_t* mapq, const uint8_t* flag) {
+    if (!ctx) return TEC_ERR_ARG;
+    if (int rc = bulk_ready(ctx, "tec_bulk_push_dev")) return rc;
+    return bulk_push_dev(ctx, n_rec, start, end, chrom, mapq, flag);
+}
+
 // Host buffers: chunks are copied on the copy stream into one of two staging slots while the
 // previous chunk is counted on the compute stream.
 extern "C" int tec_bulk_push(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const int32_t* end,
                              const uint16_t* chrom, const uint8_t* mapq, const uint8_t* flag) {
     if (!ctx) return TEC_ERR_ARG;
-    if (!ctx->bulk_active) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_push: tec_bulk_begin not called");
+    if (int rc = bulk_ready(ctx, "tec_bulk_push")) return rc;
     if (n_rec < 0 || (ctx->paired && (n_rec & 1))) TEC_FAIL(TEC_ERR_ARG, "tec_bulk_push: record count must be even in paired mode");
     if (n_rec == 0) return TEC_OK;
     if (!start || !end || !chrom || !mapq || !flag) TEC_FAIL(TEC_ERR_ARG, "tec_bulk_push: null array");
@@ -606,7 +619,7 @@ extern "C" int tec_bulk_push(tec_ctx* ctx, int64_t n_rec, const int32_t* start, 
 
 extern "C" int tec_bulk_finish(tec_ctx* ctx, int64_t* counts, int64_t* stats) {
     if (!ctx) return TEC_ERR_ARG;
-    if (!ctx->bulk_active) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_finish: tec_bulk_begin not called");
+    if (int rc = bulk_ready(ctx, "tec_bulk_finish")) return rc;
     TEC_CUDA(cudaSetDevice(ctx->device));
     const size_t ne = (size_t)ctx->idx.n_ensg;
     std::vector<int64_t> tmp(ne + TEC_BULK_NSTATS);
@@ -619,6 +632,17 @@ extern "C" int tec_bulk_finish(tec_ctx* ctx, int64_t* counts, int64_t* stats) {
 }
 
 extern "C" void* tec_bulk_counts_dev(tec_ctx* ctx) { return ctx ? (void*)ctx->d_counts : nullptr; }
+
+extern "C" int tec_bulk_keep_bank(tec_ctx* ctx, int bank) {
+    if (!ctx) return TEC_ERR_ARG;
+    if (!ctx->bulk_active || !ctx->bank_pending) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_keep_bank: no paired-end range count waits for it");
+    if (bank != 0 && bank != 1) TEC_FAIL(TEC_ERR_ARG, "tec_bulk_keep_bank: bank must be 0 or 1");
+    TEC_CUDA(cudaSetDevice(ctx->device));
+    if (bank == 1)
+        TEC_CUDA(cudaMemcpyAsync(ctx->d_counts, ctx->d_bank1, ((size_t)ctx->idx.n_ensg + TEC_BULK_NSTATS) * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+    ctx->bank_pending = false;
+    return TEC_OK;
+}
 
 extern "C" int tec_set_option(tec_ctx* ctx, const char* key, int64_t value) {
     if (!ctx || !key) return TEC_ERR_ARG;
@@ -698,6 +722,20 @@ int BamGpuBackend::deliver(int64_t n, int mode) {
     return rc ? 1 : 0;
 }
 
+// column set b into counter bank b: the bulk kernels run unchanged on d_counts, which points at bank 1 for the second push
+int BamGpuBackend::deliver_pairs(int64_t pairs0, int64_t pairs1) {
+    for (int s = 0; s < 2; s++) {
+        const int64_t n = s ? pairs1 : pairs0;
+        if (!n) continue;
+        if (s) std::swap(ctx->d_counts, ctx->d_bank1);
+        const bgzfdev::Columns& c = pairs.s[s];
+        const int rc = bulk_push_dev(ctx, 2 * n, c.start, c.end, c.chrom, c.mapq, c.flag);
+        if (s) std::swap(ctx->d_counts, ctx->d_bank1);
+        if (rc) return 1;
+    }
+    return 0;
+}
+
 static int bam_status(tec_ctx* ctx, const bamorch::Reader& r, int rc, const BamGpuBackend* be = nullptr) {
     if (rc == bamorch::OK) return TEC_OK;
     if (rc != bamorch::E_BACKEND) ctx->err = r.err;         // the backend left the CUDA text in ctx->err
@@ -760,6 +798,8 @@ extern "C" int tec_bam_count(tec_bam* b, int mode, int qual, int64_t* n_records)
         if (!ctx->sc || !ctx->sc->active) TEC_FAIL(TEC_ERR_STATE, "tec_bam_count: tec_sc_begin not called");
     } else if (!ctx->bulk_active || (ctx->paired ? 1 : 0) != mode) {
         TEC_FAIL(TEC_ERR_STATE, "tec_bam_count: tec_bulk_begin not called for this mode");
+    } else if (int st = bulk_ready(ctx, "tec_bam_count")) {
+        return st;
     }
     TEC_CUDA(cudaSetDevice(ctx->device));
     int64_t n = 0;
@@ -773,19 +813,53 @@ extern "C" int tec_bam_count_range(tec_bam* b, int mode, int qual, int64_t byte_
     tec_ctx* ctx = b->ctx;
     if (!out) TEC_FAIL(TEC_ERR_ARG, "tec_bam_count_range: out must hold TEC_BAM_RANGE_WORDS values");
     for (int i = 0; i < TEC_BAM_RANGE_WORDS; i++) out[i] = 0;
-    if (mode != bgzfdev::MODE_SE && mode != bgzfdev::MODE_SC) TEC_FAIL(TEC_ERR_ARG, "tec_bam_count_range: mode must be 0 (single end) or 2 (single cell)");
+    if (mode < 0 || mode > 2) TEC_FAIL(TEC_ERR_ARG, "tec_bam_count_range: mode must be 0 (single end), 1 (paired end) or 2 (single cell)");
     if (byte_lo < 0 || byte_hi < byte_lo) TEC_FAIL(TEC_ERR_ARG, "tec_bam_count_range: bad byte range");
     if (mode == bgzfdev::MODE_SC) {
         if (!ctx->sc || !ctx->sc->active) TEC_FAIL(TEC_ERR_STATE, "tec_bam_count_range: tec_sc_begin not called");
-    } else if (!ctx->bulk_active || ctx->paired) {
-        TEC_FAIL(TEC_ERR_STATE, "tec_bam_count_range: tec_bulk_begin not called for single-end counting");
+    } else if (!ctx->bulk_active || (ctx->paired ? 1 : 0) != mode) {
+        TEC_FAIL(TEC_ERR_STATE, "tec_bam_count_range: tec_bulk_begin not called for this mode");
+    } else if (int st = bulk_ready(ctx, "tec_bam_count_range")) {
+        return st;
     }
     TEC_CUDA(cudaSetDevice(ctx->device));
+    b->edge[0].clear();
+    b->edge[1].clear();
+    if (mode == bgzfdev::MODE_PE) {
+        // bank 1 starts as a copy of the running count; bank 0 is the running count itself
+        const size_t bytes = ((size_t)ctx->idx.n_ensg + TEC_BULK_NSTATS) * 8;
+        if (!ctx->d_bank1) TEC_CUDA(cudaMalloc(&ctx->d_bank1, bytes));
+        TEC_CUDA(cudaMemcpyAsync(ctx->d_bank1, ctx->d_counts, bytes, cudaMemcpyDeviceToDevice, ctx->stream));
+        ctx->bank_pending = true;
+    }
     bamorch::RangeResult r;
     const int rc = bamorch::decode_range(b->reader, b->be, mode, qual, ctx->opt_bam_window_blocks, (uint64_t)byte_lo, (uint64_t)byte_hi, &r);
     out[0] = r.n_records; out[1] = r.start_block; out[2] = r.start_off; out[3] = r.exit_block; out[4] = r.exit_off;
     out[5] = (int64_t)b->reader.file.size;
+    b->edge[0].swap(r.first_rec);
+    b->edge[1].swap(r.last_rec);
     return bam_status(ctx, b->reader, rc, &b->be);
+}
+
+extern "C" int tec_bam_range_record(const tec_bam* b, int which, void* buf, int64_t cap, int64_t* len) {
+    if (!b || !len || (which != 0 && which != 1)) return TEC_ERR_ARG;
+    const std::vector<uint8_t>& e = b->edge[which];
+    *len = (int64_t)e.size();
+    if (!buf) return TEC_OK;
+    if (cap < *len) {
+        b->ctx->err = "tec_bam_range_record: the buffer is smaller than the record";
+        return TEC_ERR_ARG;
+    }
+    if (!e.empty()) memcpy(buf, e.data(), e.size());
+    return TEC_OK;
+}
+
+extern "C" int tec_bam_pair_columns(tec_bam* b, const void* rec1, int64_t n1, const void* rec2, int64_t n2, int qual,
+                                    int32_t* start, int32_t* end, uint16_t* chrom, uint8_t* mapq, uint8_t* flag) {
+    if (!b || !rec1 || !rec2 || !start || !end || !chrom || !mapq || !flag) return TEC_ERR_ARG;
+    tec_ctx* ctx = b->ctx;
+    const int rc = bamorch::parse_pair(b->reader, (const uint8_t*)rec1, n1, (const uint8_t*)rec2, n2, qual, start, end, chrom, mapq, flag);
+    return bam_status(ctx, b->reader, rc);
 }
 
 extern "C" int64_t tec_bam_info(const tec_bam* b, int what) {

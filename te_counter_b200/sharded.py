@@ -3,10 +3,12 @@ One BAM counted by all GPUs of a node:
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29500 \\
         -m te_counter_b200.sharded --glb genes_tes.glb --bam in.bam --mode se -o out.tsv
+    ... --mode pe -o out.tsv
     ... --mode sc --whitelist 3M-february-2018.txt --maxcells 10000 [--strand] -o out.tsv
 
 Every rank builds the same `measureTE` the reference's bin/te_count builds (bin/te_count:77-120) and calls the same
-method; inside, the ranks split the file by byte ranges (shard.py).  Rank 0 writes the outputs, which are byte for byte
+method; inside, the ranks split the file by byte ranges (shard.py; paired end pairs records by their global index, so
+each rank keeps the counter bank of its record parity and counts the pair across its front border).  Rank 0 writes the outputs, which are byte for byte
 those of a one-GPU run.  With fewer GPUs than ranks the ranks share GPUs and talk over gloo (tests).
 """
 import argparse

@@ -186,21 +186,28 @@ class measureTE:
         label = 'reads' if paired else 'SE reads'
         more, done, next_log = True, 0, 1000000
         # One file, several ranks (torch.distributed job, one process per GPU; shard.py): every rank decodes a byte range
-        # on its GPU and the counters are summed.  Paired-end files, and files whose ranges the decoders cannot tile,
-        # are decoded by rank 0 alone; the sum is the same.
+        # on its GPU and the counters are summed; paired end keeps the counter bank of the rank's record parity and
+        # counts the pair across its front border.  Files whose ranges the decoders cannot tile are decoded by rank 0
+        # alone; the sum is the same.
         rank, world = _shard.world_info()
         in_library = _shard.join_collectives(eng) if world > 1 else False
         if world > 1:
             sharded = None
-            if not paired and _device_decoder_wanted(eng):
+            if _device_decoder_wanted(eng):
                 def open_and_bind():
                     dev = eng.bam_open(filename)
                     dev.bind(cm)
                     return dev
                 eng.bulk_begin(paired, qual)
-                sharded = _shard.count_ranges(open_and_bind, 0, qual)
+                sharded = _shard.count_ranges(open_and_bind, 1 if paired else 0, qual)
             if sharded is not None:
                 done, more = sharded[1], False
+                if paired:
+                    bank, border = sharded[2]
+                    eng.bulk_keep_bank(bank)
+                    if border is not None:
+                        eng.bulk_push(2, border['start'], border['end'], border['chrom'], border['mapq'], border['flag'])
+                    done //= 2
                 log.info('{:,} of them decoded by this rank ({} of {})'.format(sharded[0], rank, world))
             elif rank != 0:
                 eng.bulk_begin(paired, qual)                  # nothing to decode here: rank 0 reads the whole file

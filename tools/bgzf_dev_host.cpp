@@ -22,6 +22,12 @@ struct HostBackend {
     std::vector<uint8_t> o_mapq, o_flag;
     std::vector<uint32_t> o_cell;
     std::vector<uint64_t> o_umi;
+    // paired-end ranges: the two column sets of the window, and everything delivered into each
+    struct Set {
+        std::vector<int32_t> start, end;
+        std::vector<uint16_t> chrom;
+        std::vector<uint8_t> mapq, flag;
+    } p_win[2], p_out[2];
     uint32_t crc_table[256], crc_mats[bgzfdev::CRC_SHIFT_MATS * 32];
     int n_inflate_declined = 0;
     int force_decline_every = 0;                // test hook: pretend the block-parallel inflate declined every k-th block
@@ -108,6 +114,51 @@ struct HostBackend {
         }
         return 0;
     }
+    int parse_pairs(const bamorch::BlockChain* ch, const int64_t* base, int nb, int64_t n, int64_t g0, int qual, const bamorch::Reader& r,
+                    int* err, int64_t* err_rec) {
+        std::vector<int64_t> rec_off((size_t)n);
+        for (int b = 0; b < nb; b++) {          // bam_list_kernel: one CUDA thread per b
+            int64_t p = ch[b].start;
+            for (uint32_t i = 0; i < ch[b].count; i++) {
+                rec_off[(size_t)(base[b] + i)] = p;
+                p += 4 + (int64_t)bgzfdev::ld32(ubuf.data() + p);
+            }
+        }
+        bgzfdev::Columns sets[2];
+        for (int s = 0; s < 2; s++) {
+            Set& w = p_win[s];
+            w.start.resize((size_t)n); w.end.resize((size_t)n); w.chrom.resize((size_t)n); w.mapq.resize((size_t)n); w.flag.resize((size_t)n);
+            sets[s] = bgzfdev::Columns{w.start.data(), w.end.data(), w.chrom.data(), w.mapq.data(), w.flag.data(), nullptr, nullptr};
+        }
+        const bgzfdev::ParseCtx pc = r.host_parse_ctx(qual);
+        uint64_t first_err = ~uint64_t(0);
+        for (int64_t i = 0; i + 1 < n; i++) {   // bam_parse_pairs_kernel: one CUDA thread per adjacent pair
+            const int e = bgzfdev::parse_adjacent_pair(ubuf.data(), rec_off.data(), i, g0, pc, sets);
+            if (e) first_err = std::min(first_err, ((uint64_t)i << 8) | (uint64_t)e);
+        }
+        *err = 0;
+        if (first_err != ~uint64_t(0)) {
+            *err = (int)(first_err & 0xFF);
+            *err_rec = (int64_t)(first_err >> 8);
+        }
+        return 0;
+    }
+    int deliver_pairs(int64_t pairs0, int64_t pairs1) {
+        for (int s = 0; s < 2; s++) {
+            const size_t n = 2 * (size_t)(s ? pairs1 : pairs0);
+            Set &w = p_win[s], &o = p_out[s];
+            o.start.insert(o.start.end(), w.start.begin(), w.start.begin() + n);
+            o.end.insert(o.end.end(), w.end.begin(), w.end.begin() + n);
+            o.chrom.insert(o.chrom.end(), w.chrom.begin(), w.chrom.begin() + n);
+            o.mapq.insert(o.mapq.end(), w.mapq.begin(), w.mapq.begin() + n);
+            o.flag.insert(o.flag.end(), w.flag.begin(), w.flag.begin() + n);
+        }
+        return 0;
+    }
+    int fetch(int64_t at, uint8_t* dst, size_t n) {
+        memcpy(dst, ubuf.data() + at, n);
+        return 0;
+    }
     int deliver(int64_t n, int mode) {
         o_start.insert(o_start.end(), c_start.begin(), c_start.begin() + n);
         o_end.insert(o_end.end(), c_end.begin(), c_end.begin() + n);
@@ -125,6 +176,7 @@ struct HostBackend {
 struct Session {
     bamorch::Reader reader;
     HostBackend be;
+    std::vector<uint8_t> edge[2];               // first / last record of the last paired-end range
 };
 
 }  // namespace
@@ -164,7 +216,38 @@ int bgzfdev_decode_range(void* h, int mode, int qual, int window_blocks, int64_t
     const int rc = bamorch::decode_range(s->reader, s->be, mode, qual, window_blocks, (uint64_t)lo, (uint64_t)hi, &r);
     out[0] = r.n_records; out[1] = r.start_block; out[2] = r.start_off; out[3] = r.exit_block; out[4] = r.exit_off;
     out[5] = (int64_t)s->reader.file.size;
+    s->edge[0].swap(r.first_rec);
+    s->edge[1].swap(r.last_rec);
     return rc;
+}
+
+// paired-end range: rows of column set `bank` delivered so far, and a copy of them
+int64_t bgzfdev_set_rows(void* h, int bank) { return (int64_t)((Session*)h)->be.p_out[bank].start.size(); }
+void bgzfdev_fetch_set(void* h, int bank, int32_t* start, int32_t* end, uint16_t* chrom, uint8_t* mapq, uint8_t* flag) {
+    const HostBackend::Set& o = ((Session*)h)->be.p_out[bank];
+    const size_t n = o.start.size();
+    if (!n) return;
+    memcpy(start, o.start.data(), n * 4);
+    memcpy(end, o.end.data(), n * 4);
+    memcpy(chrom, o.chrom.data(), n * 2);
+    memcpy(mapq, o.mapq.data(), n);
+    memcpy(flag, o.flag.data(), n);
+}
+
+// tec_bam_range_record of the host decoder: first (0) / last (1) record of the last paired-end range
+int bgzfdev_range_record(void* h, int which, void* buf, int64_t cap, int64_t* len) {
+    const std::vector<uint8_t>& e = ((Session*)h)->edge[which];
+    *len = (int64_t)e.size();
+    if (!buf) return 0;
+    if (cap < *len) return bamorch::E_ARG;
+    if (!e.empty()) memcpy(buf, e.data(), e.size());
+    return 0;
+}
+
+// tec_bam_pair_columns of the host decoder
+int bgzfdev_pair_columns(void* h, const void* rec1, int64_t n1, const void* rec2, int64_t n2, int qual, int32_t* start, int32_t* end,
+                         uint16_t* chrom, uint8_t* mapq, uint8_t* flag) {
+    return bamorch::parse_pair(((Session*)h)->reader, (const uint8_t*)rec1, n1, (const uint8_t*)rec2, n2, qual, start, end, chrom, mapq, flag);
 }
 
 // copies the delivered columns out (cell / umi only for single cell)
