@@ -132,7 +132,10 @@ int tec_trim(tec_ctx* ctx);
  * Part 3, 1 cell table), "sc_pack_umi" (2-bit UMI sort keys when possible).
  * tec_get_info: "has_stab", "stab_bytes", "has_sc_stab", "sc_stab_bytes", "n_sm", "n_features",
  * "stab_primary", "stab_overflow", "stab_entries", "last_slow_units", "last_deferred_units", "last_left_units"
- * (deferred units the two-sector kernel left for the second pass), "stab_refused";
+ * (deferred units the two-sector kernel left for the second pass), "stab_refused",
+ * "sc_last_sort" (how the last tec_sc_finalize grouped the survivors by (cell, UMI): 1 one packed 64-bit key per
+ * survivor sorted by csrc/radix.cuh, 2 library sorts on 2-bit-per-character UMI keys, 3 library sorts on the 3-bit
+ * UMI codes; 0 nothing was sorted), "sc_last_sort_passes" (radix passes of that packed sort, 0 on the other routes);
  * -1 for unknown keys. */
 int tec_set_option(tec_ctx* ctx, const char* key, int64_t value);
 int64_t tec_get_info(tec_ctx* ctx, const char* key);

@@ -180,6 +180,10 @@ struct tec_ctx {
                                           // (measured SLOWER at 1 B records: 167.6 vs 156.0 ms per step, gpurun_out/r02w; 2 = also on small inputs, tests)
     int opt_sc_pack_umi = 1;              // single cell: 2-bit UMI sort keys when every UMI is fixed-length ACGT
     int opt_sc_algo = -1;                 // -1 auto, 0 exact search only, 1 cell table
+    // single cell, last finalize (tec_get_info): 1 packed keys + radix.cuh, 2 library sorts on 2-bit UMI keys, 3 library sorts
+    // on 3-bit UMI codes, 0 nothing sorted; and the radix passes of the packed sort
+    int sc_last_sort = 0;
+    int sc_last_sort_passes = 0;
     int opt_bam_lanes = 1;                // BGZF blocks decoded per warp by the inflate kernel (1..32): the streams of a warp
                                           // diverge on every symbol; measured 201 ms (1) / 206 (2) / 241 (8) / 398 (32) per 3.7 GB
     int opt_bam_window_blocks = 65536;    // BGZF blocks decoded per pass by tec_bam_count (one thread each)

@@ -336,19 +336,28 @@ static cudaError_t rdx_pass(const K* keys_in, const u32* vals_in, K* keys_out, u
 }
 #define RDX_LAUNCHES_PER_PASS 5
 
+// digit widths of a sort over `total` key bits (at most 64): ceil(total / max_bits) passes whose widths differ by at most
+// one, wider passes first; returns the number of passes
+static inline int rdx_digit_widths(int total, int widths[64]) {
+    total = std::min(64, std::max(0, total));
+    const int max_bits = std::min(RDX_MAX_BITS, std::max(1, g_rdx_max_bits));
+    const int passes = (total + max_bits - 1) / max_bits;
+    for (int i = 0, done = 0; i < passes; ++i) done += widths[i] = (total - done + (passes - i) - 1) / (passes - i);
+    return passes;
+}
+
 // stable sort on key bits [bit_lo, bit_hi) in ceil((bit_hi - bit_lo) / 11) passes of equal width, ping-pong between
 // (keys_a, vals_a) and (keys_b, vals_b); *in_b says where the result is.  n < 2^32 - 2^13.
 template <class K, bool HAS_VALUES>
 static cudaError_t rdx_sort(K* keys_a, u32* vals_a, K* keys_b, u32* vals_b, int64_t n, int bit_lo, int bit_hi, int n_sm,
                             u32* scratch, cudaStream_t st, bool* in_b, int* n_passes = nullptr) {
-    const int total = std::max(0, bit_hi - bit_lo);
-    const int max_bits = std::min(RDX_MAX_BITS, std::max(1, g_rdx_max_bits));
-    const int passes = (total + max_bits - 1) / max_bits;
+    int widths[64];
+    const int passes = rdx_digit_widths(bit_hi - bit_lo, widths);
     const RdxPlan plan = rdx_plan(n, n_sm);
     bool flip = false;
     int done = 0;
     for (int i = 0; i < passes; ++i) {
-        const int bits = (total - done + (passes - i) - 1) / (passes - i);
+        const int bits = widths[i];
         cudaError_t e = flip ? rdx_pass<K, HAS_VALUES>(keys_b, vals_b, keys_a, vals_a, n, bit_lo + done, bits, plan, scratch, st)
                              : rdx_pass<K, HAS_VALUES>(keys_a, vals_a, keys_b, vals_b, n, bit_lo + done, bits, plan, scratch, st);
         if (e != cudaSuccess) return e;

@@ -1238,6 +1238,7 @@ extern "C" int tec_sc_finalize(tec_ctx* ctx, int64_t bundle_keys, int64_t maxcel
         TEC_CUDA(cudaMemcpyAsync(d_ensg_of_slot, ctx->ensg_of_slot.data(), ctx->ensg_of_slot.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
     u64* pairs_sorted = nullptr;
     u32 h_npairs = 0;
+    ctx->sc_last_sort = ctx->sc_last_sort_passes = 0;
     if (N > 0 || s->world > 1) {          // with several ranks every rank walks the same sequence of collectives
         // ---- key groups: survivors in (cell, UMI, file position) order
         u64* d_or = s->d_n + 1;                 // kept up to date by the pushes
@@ -1281,6 +1282,8 @@ extern "C" int tec_sc_finalize(tec_ctx* ctx, int64_t bundle_keys, int64_t maxcel
                 int n_pass = 0;
                 TEC_CUDA((rdx_sort<u64, true>(ka, va, kb, vb, N, cs_bits, cs_bits + 2 * umi_len + cell_bits, ctx->n_sm, scratch, ctx->stream, &in_b, &n_pass)));
                 ctx->launches += RDX_LAUNCHES_PER_PASS * n_pass;
+                ctx->sc_last_sort = 1;
+                ctx->sc_last_sort_passes = n_pass;
                 const u64* skey = in_b ? kb : ka;
                 perm = in_b ? vb : va;
                 u32* free_v = in_b ? va : vb;                 // the other half of the ping-pong: free from here on
@@ -1344,6 +1347,7 @@ extern "C" int tec_sc_finalize(tec_ctx* ctx, int64_t bundle_keys, int64_t maxcel
                 rc = sc_sort_pairs(ctx, s->umi, uk, iota, perm1, N, b0, b1);
                 if (rc) return rc;
             }
+            if (N > 0) ctx->sc_last_sort = packed ? 2 : 3;      // a rank without survivors sorts nothing
             A.release(uk); uk = nullptr;
             TEC_CUDA(A.get(&ck, (size_t)N));
             TEC_CUDA(A.get(&scell, (size_t)N));

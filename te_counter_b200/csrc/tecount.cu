@@ -699,6 +699,8 @@ extern "C" int64_t tec_get_info(tec_ctx* ctx, const char* key) {
     if (k == "has_sc_stab") return ctx->idx.has_sc_stab ? 1 : 0;
     if (k == "sc_stab_bytes") return (int64_t)ctx->idx.sc_stab_bytes;
     if (k == "n_sm") return ctx->n_sm;
+    if (k == "sc_last_sort") return ctx->sc_last_sort;
+    if (k == "sc_last_sort_passes") return ctx->sc_last_sort_passes;
     if (k == "n_features") return ctx->idx.n_feat;
     if (k == "last_slow_units") {          // units the last fast-kernel launch handed to the exact kernel
         u32 n = 0;

@@ -257,3 +257,158 @@ def test_header_over_many_blocks_empty_blocks_and_no_references(lib, tmp_path):
     assert rc == 0 and len(got["start"]) == 500
     for k in want:
         assert np.array_equal(want[k], got[k]), k
+
+
+# ---- the whitelist hash table at the size of a 10x v2 whitelist (737 280 barcodes of 16 bases + "-1")
+
+def wl_hash(bc):
+    """bgzf_dev.h wl_hash restated over equal-length barcodes: uint8 array (n, length) -> uint64 (n,)."""
+    h = np.full(len(bc), 0xcbf29ce484222325, np.uint64)
+    for i in range(bc.shape[1]):
+        h = (h ^ bc[:, i]) * np.uint64(0x100000001b3)
+    h ^= h >> np.uint64(29)
+    h *= np.uint64(0xbf58476d1ce4e5b9)
+    return h ^ (h >> np.uint64(32))
+
+
+def wl_table(hashes):
+    """bam_orch.h set_whitelist: open addressing in id order.  (capacity, slot of every id)"""
+    cap = 16
+    while cap < 2 * len(hashes) + 2:
+        cap <<= 1
+    slot, at = [0] * cap, []
+    for h in (hashes & np.uint64(cap - 1)).tolist():
+        while slot[h]:
+            h = (h + 1) & (cap - 1)
+        slot[h] = len(at) + 1
+        at.append(h)
+    return cap, np.array(at), slot
+
+
+def _barcodes(v):
+    """16-base barcodes + '-1' of the 32-bit values v, as an uint8 array (n, 18)"""
+    b = np.frombuffer(b"ACGT", np.uint8)[(v.astype(np.uint32)[:, None] >> (2 * np.arange(15, -1, -1, dtype=np.uint32))) & np.uint32(3)]
+    return np.concatenate([b, np.tile(np.frombuffer(b"-1", np.uint8), (len(v), 1))], axis=1)
+
+
+def _strings(a):
+    return [bytes(x).decode() for x in a]
+
+
+def _variants(s):
+    """the prefixes and one-character extensions of a barcode that a lookup without the length test would confuse with it"""
+    return [s[:-1], s[:16], s + "A"]
+
+
+def tenx_whitelist(seed=3, n=737_280):
+    """A whitelist of n barcodes and the barcodes a lookup can trip over: whitelisted ones whose probe chain wraps past
+    the table's last slot, absent ones whose chain starts in that full run, one-base neighbours of whitelisted ones,
+    and prefixes and extensions of whitelisted barcodes.  For six whitelisted barcodes a prefix or extension has the
+    same home slot, so its probe chain passes the barcode and only the length test in wl_find tells them apart."""
+    rng = np.random.default_rng(seed)
+    n_tail, n_same = 4, 6
+    v = np.unique(rng.integers(0, 1 << 32, n + 200_000, dtype=np.uint64))
+    v = rng.permutation(v)[:n - n_tail - n_same]
+    cap = 16
+    while cap < 2 * n + 2:
+        cap <<= 1
+    m = np.uint64(cap - 1)
+    tail, same = set(), set()                               # not yet whitelisted: home in the last two slots / shared with a variant
+    while len(tail) < 2 * n_tail or len(same) < n_same:
+        c = rng.integers(0, 1 << 32, 1 << 20, dtype=np.uint64)
+        c = c[~np.isin(c, v)]
+        b = _barcodes(c)
+        home = wl_hash(b) & m
+        tail |= set(c[home >= cap - 2].tolist())
+        ext = np.concatenate([b, np.full((len(b), 1), ord("A"), np.uint8)], axis=1)
+        hit = ((wl_hash(b[:, :17]) & m) == home) | ((wl_hash(b[:, :16]) & m) == home) | ((wl_hash(ext) & m) == home)
+        same |= set(c[hit].tolist())
+    same = sorted(same - tail)[:n_same]
+    tail = sorted(tail)[:2 * n_tail]
+    same_s = _strings(_barcodes(np.array(same, np.uint64)))
+    wl = sorted(_strings(_barcodes(np.array(list(v) + tail[:n_tail] + same, np.uint64))))
+    assert len(wl) == n
+    absent_tail = _strings(_barcodes(np.array(tail[n_tail:], np.uint64)))
+    a = np.frombuffer("".join(wl).encode(), np.uint8).reshape(len(wl), 18)
+    cap_, at, slot = wl_table(wl_hash(a))
+    assert cap_ == cap
+    home = (wl_hash(a) & m).astype(np.int64)
+    wrapped = [wl[i] for i in np.flatnonzero(at < home)]
+    assert len(wrapped) >= 2 and all(slot[cap - 2:])        # chains run over the last slot
+    wls = set(wl)
+    shadow = []                                             # absent variants whose probe chain passes their barcode's slot
+    for s in same_s:
+        i = wl.index(s)
+        for p in _variants(s):
+            h = int(wl_hash(np.frombuffer(p.encode(), np.uint8)[None, :])[0] & m)
+            while slot[h] and h != at[i]:
+                h = (h + 1) & (cap - 1)
+            if h == at[i] and p not in wls:
+                shadow.append(p)
+    assert len(shadow) >= n_same
+    near = []
+    for i in rng.integers(0, len(wl), 300).tolist():
+        s, j = wl[i], int(rng.integers(16))
+        c = s[:j] + "ACGT"[("ACGT".index(s[j]) + 1 + int(rng.integers(3))) % 4] + s[j + 1:]
+        if c not in wls:
+            near.append(c)
+    part = []
+    for s in [wl[i] for i in rng.integers(0, len(wl), 100).tolist()] + wrapped:
+        part += [x for x in _variants(s) + [s + "1"] if x not in wls]
+    return wl, {"wrapped": wrapped, "absent_tail": absent_tail, "near": near, "prefix_extension": part,
+                "same_home": shadow + same_s}
+
+
+def tenx_records(wl, groups, n, seed):
+    """single-cell records whose CB tags cycle through whitelisted barcodes and every group of tenx_whitelist"""
+    rng = np.random.default_rng(seed)
+    kinds = [wl] * 5 + [groups[k] for k in ("wrapped", "absent_tail", "near", "prefix_extension", "same_home")]
+    chroms = ["chr1", "chr2", "2", "chrX", "scaffold7"]
+    recs = []
+    for i in range(n):
+        pool = kinds[i % len(kinds)]
+        start = int(rng.integers(0, 150000))
+        recs.append({"chrom": chroms[int(rng.integers(len(chroms)))], "start": start, "end": start + 60,
+                     "flag": 16 * int(rng.integers(2)), "mapq": 60, "CB": pool[int(rng.integers(len(pool)))],
+                     "UB": "".join("ACGT"[int(x)] for x in rng.integers(0, 4, 12)), "name": "r%d" % i})
+    return recs
+
+
+def test_wl_hash_restatement(lib):
+    lib.bgzfdev_wl_hash.restype = ctypes.c_uint64
+    lib.bgzfdev_wl_hash.argtypes = [ctypes.c_char_p, ctypes.c_uint32]
+    rng = np.random.default_rng(8)
+    for length in (0, 1, 2, 7, 8, 16, 18, 19, 40):
+        a = rng.integers(0, 256, (64, length), dtype=np.uint8)
+        a[:8] = np.frombuffer(b"ACGT", np.uint8)[rng.integers(0, 4, (8, length))]
+        want = [lib.bgzfdev_wl_hash(bytes(x), length) for x in a]
+        assert wl_hash(a).tolist() == want, length
+
+
+@pytest.fixture(scope="module")
+def tenx():
+    return tenx_whitelist()
+
+
+@pytest.mark.parametrize("window_blocks", [1, 5])
+def test_10x_whitelist_lookups(lib, tmp_path, tenx, window_blocks):
+    """The block-parallel decoder's whitelist table at 737 280 barcodes against libtecbam and the dictionary lookup:
+    probe chains that wrap past the last slot, absent barcodes that walk a full chain, one-base neighbours, prefixes
+    and extensions of whitelisted barcodes, among them ones whose probe chain passes the barcode they extend."""
+    wl_list, groups = tenx
+    recs = tenx_records(wl_list, groups, 6000, 5)
+    path = str(tmp_path / "x.bam")
+    write_bam(path, recs, block=3000)
+    wlf = tmp_path / "wl.txt"
+    wlf.write_text("".join(w + "\n" for w in wl_list))
+    wl = reads.Whitelist(str(wlf))
+    idx = H.load_index("idx_rand_a.glb")
+    want = _native(path, "sc", reads.ChromMap(idx.chrom_keys), wl, 20)
+    rc, msg, got = _decode(lib, path, "sc", reads.ChromMap(idx.chrom_keys), wl, 20, window_blocks)
+    assert rc == 0, msg
+    for k in want:
+        assert np.array_equal(want[k], got[k]), k
+    ids = np.array([wl.barcode_to_id.get(r["CB"], reads.CELL_INVALID) for r in recs], np.uint32)
+    assert np.array_equal(got["cell"], ids)
+    n_group = {k: sum(r["CB"] in set(v) for r in recs) for k, v in groups.items()}
+    assert min(n_group.values()) > 100 and (ids != reads.CELL_INVALID).sum() == sum(r["CB"] in wl.barcode_to_id for r in recs)

@@ -195,3 +195,36 @@ def test_htslib_shaped_files_on_the_device(engine, tmp_path, name):
     assert np.array_equal(got[0], counts) and np.array_equal(got[1], st)
     oc, _ = te_oracle.bulk_count(H.oracle_index(idx), False, 20, *[want[k].tolist() for k in ("start", "end", "chrom", "mapq", "flag")])
     assert counts.tolist() == oc and sum(oc) > 0
+
+
+@pytest.fixture(scope="module")
+def tenx():
+    from test_bgzf_dev_cpu import tenx_whitelist
+    return tenx_whitelist()
+
+
+@pytest.mark.parametrize("window_blocks", [1, 5])
+def test_device_decoder_10x_whitelist(engine, tmp_path, tenx, window_blocks):
+    """The device whitelist table at 737 280 barcodes (16 bases + '-1'): probe chains that wrap past the last slot,
+    absent barcodes that walk a full chain, one-base neighbours, prefixes and extensions (some of them with the home
+    slot of the barcode they extend), against libtecbam."""
+    from test_bgzf_dev_cpu import tenx_records
+    wl_list, groups = tenx
+    path = str(tmp_path / "x.bam")
+    write_bam(path, tenx_records(wl_list, groups, 6000, 5), block=3000)
+    wlf = tmp_path / "wl.txt"
+    wlf.write_text("".join(w + "\n" for w in wl_list))
+    wl = reads.Whitelist(str(wlf))
+    idx = H.load_index("idx_rand_a.glb")
+    engine.upload_index(idx)
+    want = _host_run(engine, path, "sc", idx, wl, 20)
+    engine.set_option("bam_window_blocks", window_blocks)
+    try:
+        n, info, got = _device_run(engine, path, "sc", idx, wl, 20)
+    finally:
+        engine.set_option("bam_window_blocks", 32768)
+    assert n == 6000 and info["host_inflated_blocks"] == 0
+    assert len(want) == len(got)
+    for a, b in zip(want, got):
+        assert np.array_equal(a, b)
+    assert want[5][_lib.SS_INVALID_BARCODE] > 1000 and want[5][_lib.SS_VALID] > 1000

@@ -278,6 +278,9 @@ uint32_t bgzfdev_crc32_lanes(const void* p, int64_t n) {
     return c ^ 0xFFFFFFFFu;
 }
 
+// the whitelist hash of the decoder (bgzf_dev.h), for holding its numpy restatement against it
+uint64_t bgzfdev_wl_hash(const void* p, uint32_t n) { return bgzfdev::wl_hash((const uint8_t*)p, n); }
+
 // the block inflate alone, for holding it against zlib
 int bgzfdev_inflate_raw(const void* in, int64_t n_in, void* out, int64_t n_out) {
     std::vector<uint8_t> scratch(bgzfdev::SCRATCH_STRIDE);
