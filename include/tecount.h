@@ -259,6 +259,16 @@ int tec_sc_matrix_text(tec_ctx *ctx, int64_t n_rows, const uint32_t *cells, cons
                        const int64_t *bc_off, int64_t *n_bytes);
 int tec_sc_matrix_read(tec_ctx *ctx, int64_t offset, int64_t n, char *out);
 
+/*
+ * The cell x feature matrix of sc_save_result as the text of a Matrix Market file, 10x orientation: one row per feature
+ * (ensg id order = the dense TSV's columns), one column per given cell (cells[k] = whitelist id of column k, each at
+ * most once; normally tec_sc_select's order).  Text = "%%MatrixMarket matrix coordinate integer general\n",
+ * "<n_ensg> <n_cols> <nnz>\n", then one line "<ensg + 1> <k + 1> <count>\n" per non-zero, ascending in (k, ensg).
+ * *nnz = entries written, *n_bytes = text length.  The text replaces the one tec_sc_matrix_text keeps and is read
+ * with tec_sc_matrix_read.  n_cols == 0 gives the two header lines only.
+ */
+int tec_sc_matrix_mtx(tec_ctx *ctx, int64_t n_cols, const uint32_t *cells, int64_t *nnz, int64_t *n_bytes);
+
 /* ---- BAM file -> counting path, decoded on the device (SURVEY.md 8f-1; te_count.py:65-98, :190-214, :351-438)
  *
  * The same job as libtecbam (include/tecbam.h: BGZF inflate, record split, fields -> SoA columns, same

@@ -69,6 +69,7 @@ SIGNATURES = {
     "tec_bam_info": (ctypes.c_int64, [_vp, ctypes.c_int]),
     "tec_sc_matrix_text": (ctypes.c_int, [_vp, ctypes.c_int64, _c_u32p, ctypes.c_char_p, _c_i64p, _c_i64p]),
     "tec_sc_matrix_read": (ctypes.c_int, [_vp, ctypes.c_int64, ctypes.c_int64, _vp]),
+    "tec_sc_matrix_mtx": (ctypes.c_int, [_vp, ctypes.c_int64, _c_u32p, _c_i64p, _c_i64p]),
     "tec_sc_set_collective": (ctypes.c_int, [_vp, _vp, _vp, ctypes.c_int, ctypes.c_int]),
     "tec_sc_survivors": (ctypes.c_int, [_vp, _c_i64p]),
     "tec_sc_partition_dev": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int64, _c_i64p, ctypes.POINTER(_vp)]),
@@ -527,8 +528,18 @@ class Engine:
                                                  ctypes.cast(off.ctypes.data, _c_i64p), ctypes.byref(n)))
         return n.value
 
+    def sc_matrix_mtx(self, cells):
+        """Builds the matrix as Matrix Market text on the device (include/tecount.h tec_sc_matrix_mtx): one row per
+        feature, one column per given whitelist id, in that order.  Returns (non-zeros, bytes); stream it with
+        sc_matrix_write."""
+        cells = np.ascontiguousarray(cells, dtype=np.uint32)
+        nnz, n = ctypes.c_int64(0), ctypes.c_int64(0)
+        self._check(self._lib.tec_sc_matrix_mtx(self._h, len(cells), ctypes.cast(cells.ctypes.data, _c_u32p),
+                                                ctypes.byref(nnz), ctypes.byref(n)))
+        return nnz.value, n.value
+
     def sc_matrix_write(self, fh, n_bytes, chunk=1 << 26):
-        """Streams the text built by sc_matrix_text into the binary file object `fh`."""
+        """Streams the text built by sc_matrix_text or sc_matrix_mtx into the binary file object `fh`."""
         if getattr(self, "_text_buf", None) is None or len(self._text_buf) < min(chunk, max(1, n_bytes)):
             self._text_buf = self.pinned(min(chunk, max(1, n_bytes)), np.uint8)
         buf = self._text_buf

@@ -1109,7 +1109,7 @@ extern "C" int tec_sc_survivors(tec_ctx* ctx, int64_t* n) {
     return TEC_OK;
 }
 
-static int sc_excl_sum(tec_ctx* ctx, u32* in, u32* out, int64_t n);
+template <class T> static int sc_excl_sum(tec_ctx* ctx, T* in, T* out, int64_t n);
 
 // Pack the survivors as 32-byte records grouped by owner rank (cell % world), file order kept inside a
 // group; counts[world] on the host.  The packed buffer lives until the next call / import.
@@ -1204,7 +1204,9 @@ static int sc_incl_scan(tec_ctx* ctx, T* v, int64_t n, Op op) {
     return TEC_OK;
 }
 
-static int sc_excl_sum(tec_ctx* ctx, u32* in, u32* out, int64_t n) {
+// T = u32, or u64 for byte offsets that can pass 4 GiB (sc_mtx.cuh)
+template <class T>
+static int sc_excl_sum(tec_ctx* ctx, T* in, T* out, int64_t n) {
     size_t tb = 0;
     TEC_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tb, in, out, (int)n, ctx->stream));
     int rc = sc_cub_tmp(ctx, tb);

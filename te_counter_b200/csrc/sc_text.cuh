@@ -106,6 +106,47 @@ static void sc_text_free(tec_ctx* ctx) {
     s->text_bytes = 0;
 }
 
+// The rows of both matrix texts (this file and sc_mtx.cuh): the rank of each listed cell (TEC_ERR_ARG for an id outside
+// the whitelist or listed twice), the triples stably sorted by that rank -- unlisted cells last, ensg ascending inside a
+// rank, so the listed cells' triples are ascending in (rank, ensg) -- and row_ptr[r] = first sorted position of rank r
+// for r in [0, n_rows + 1].  *n_sel = row_ptr[n_rows] = triples of the listed cells.  The buffers live in A.
+static int sc_text_rows(tec_ctx* ctx, ScArena& A, const char* who, int64_t n_rows, const uint32_t* cells,
+                        u32** skey_out, u32** sval_out, u32** row_ptr_out, int64_t* n_sel) {
+    ScState* s = ctx->sc;
+    const int64_t T = s->n_triples;
+    u32 *d_cells, *rank, *key, *val, *skey, *sval, *row_ptr;
+    int* d_bad;
+    TEC_CUDA(A.get(&d_cells, (size_t)n_rows));
+    TEC_CUDA(A.get(&rank, (size_t)s->n_wl));
+    TEC_CUDA(A.get(&key, (size_t)T));
+    TEC_CUDA(A.get(&val, (size_t)T));
+    TEC_CUDA(A.get(&skey, (size_t)T));
+    TEC_CUDA(A.get(&sval, (size_t)T));
+    TEC_CUDA(A.get(&row_ptr, (size_t)n_rows + 2));
+    TEC_CUDA(A.get(&d_bad, 1));
+    TEC_CUDA(cudaMemcpyAsync(d_cells, cells, (size_t)n_rows * 4, cudaMemcpyHostToDevice, ctx->stream));
+    TEC_CUDA(cudaMemsetAsync(d_bad, 0, 4, ctx->stream));
+    TEC_CUDA(cudaMemsetAsync(rank, 0xFF, (size_t)s->n_wl * 4, ctx->stream));
+    sc_text_rank_kernel<<<SC_GRID(n_rows)>>>(n_rows, d_cells, rank, s->n_wl, d_bad);
+    if (T) {
+        sc_text_rowkey_kernel<<<SC_GRID(T)>>>(T, s->t_cell, rank, (u32)n_rows, key, val);
+        int rc = sc_sort_pairs(ctx, key, skey, val, sval, T, 0, ceil_log2_i64(n_rows + 2));
+        if (rc) return rc;
+    }
+    sc_text_rowptr_kernel<<<SC_GRID(T + 1)>>>(T, skey, (u32)n_rows, row_ptr);
+    u32 h_ptr = 0;
+    int h_bad = 0;
+    TEC_CUDA(cudaMemcpyAsync(&h_ptr, row_ptr + n_rows, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    TEC_CUDA(cudaMemcpyAsync(&h_bad, d_bad, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    TEC_CUDA(cudaStreamSynchronize(ctx->stream));
+    if (h_bad) TEC_FAIL(TEC_ERR_ARG, std::string(who) + ": cell id outside the whitelist or listed twice");
+    *skey_out = skey;
+    *sval_out = sval;
+    *row_ptr_out = row_ptr;
+    *n_sel = h_ptr;
+    return TEC_OK;
+}
+
 extern "C" int tec_sc_matrix_text(tec_ctx* ctx, int64_t n_rows, const uint32_t* cells, const char* barcodes,
                                   const int64_t* bc_off, int64_t* n_bytes) {
     if (!ctx) return TEC_ERR_ARG;
@@ -119,47 +160,23 @@ extern "C" int tec_sc_matrix_text(tec_ctx* ctx, int64_t n_rows, const uint32_t* 
     if (!n_rows) return TEC_OK;
     for (int64_t r = 0; r < n_rows; ++r)
         if (bc_off[r + 1] < bc_off[r] || bc_off[0] != 0) TEC_FAIL(TEC_ERR_ARG, "tec_sc_matrix_text: barcode offsets must ascend from 0");
-    const int64_t n_ensg = ctx->idx.n_ensg, T = s->n_triples, bc_bytes = bc_off[n_rows];
+    const int64_t n_ensg = ctx->idx.n_ensg, bc_bytes = bc_off[n_rows];
     if (bc_bytes && !barcodes) TEC_FAIL(TEC_ERR_ARG, "tec_sc_matrix_text: null barcodes");
     ScArena A(ctx->cache);
-    u32 *d_cells, *rank, *key, *val, *skey, *sval, *row_ptr, *extra, *E;
+    u32 *skey, *sval, *row_ptr, *extra, *E;
     int64_t* d_off;
     char* d_bc;
-    int* d_bad;
-    TEC_CUDA(A.get(&d_cells, (size_t)n_rows));
-    TEC_CUDA(A.get(&rank, (size_t)s->n_wl));
-    TEC_CUDA(A.get(&key, (size_t)T));
-    TEC_CUDA(A.get(&val, (size_t)T));
-    TEC_CUDA(A.get(&skey, (size_t)T));
-    TEC_CUDA(A.get(&sval, (size_t)T));
-    TEC_CUDA(A.get(&row_ptr, (size_t)n_rows + 2));
     TEC_CUDA(A.get(&d_off, (size_t)n_rows + 1));
     TEC_CUDA(A.get(&d_bc, (size_t)bc_bytes));
-    TEC_CUDA(A.get(&d_bad, 1));
-    TEC_CUDA(cudaMemcpyAsync(d_cells, cells, (size_t)n_rows * 4, cudaMemcpyHostToDevice, ctx->stream));
     TEC_CUDA(cudaMemcpyAsync(d_off, bc_off, (size_t)(n_rows + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
     if (bc_bytes) TEC_CUDA(cudaMemcpyAsync(d_bc, barcodes, (size_t)bc_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    TEC_CUDA(cudaMemsetAsync(d_bad, 0, 4, ctx->stream));
-    TEC_CUDA(cudaMemsetAsync(rank, 0xFF, (size_t)s->n_wl * 4, ctx->stream));
-    sc_text_rank_kernel<<<SC_GRID(n_rows)>>>(n_rows, d_cells, rank, s->n_wl, d_bad);
     int64_t n_sel = 0;
-    if (T) {
-        sc_text_rowkey_kernel<<<SC_GRID(T)>>>(T, s->t_cell, rank, (u32)n_rows, key, val);
-        int rc = sc_sort_pairs(ctx, key, skey, val, sval, T, 0, ceil_log2_i64(n_rows + 2));
-        if (rc) return rc;
-    }
-    sc_text_rowptr_kernel<<<SC_GRID(T + 1)>>>(T, skey, (u32)n_rows, row_ptr);
-    u32 h_ptr = 0;
-    int h_bad = 0;
-    TEC_CUDA(cudaMemcpyAsync(&h_ptr, row_ptr + n_rows, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    TEC_CUDA(cudaMemcpyAsync(&h_bad, d_bad, 4, cudaMemcpyDeviceToHost, ctx->stream));
-    TEC_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (h_bad) TEC_FAIL(TEC_ERR_ARG, "tec_sc_matrix_text: cell id outside the whitelist or listed twice");
-    n_sel = h_ptr;
+    int rc = sc_text_rows(ctx, A, "tec_sc_matrix_text", n_rows, cells, &skey, &sval, &row_ptr, &n_sel);
+    if (rc) return rc;
     TEC_CUDA(A.get(&extra, (size_t)n_sel + 1));
     TEC_CUDA(A.get(&E, (size_t)n_sel + 1));
     sc_text_extra_kernel<<<SC_GRID(n_sel + 1)>>>(n_sel, sval, s->t_count, extra);
-    int rc = sc_excl_sum(ctx, extra, E, n_sel + 1);
+    rc = sc_excl_sum(ctx, extra, E, n_sel + 1);
     if (rc) return rc;
     u32 h_extra = 0;
     TEC_CUDA(cudaMemcpyAsync(&h_extra, E + n_sel, 4, cudaMemcpyDeviceToHost, ctx->stream));

@@ -7,6 +7,7 @@
 #include "sc.cuh"
 #include "sc_comm.cuh"
 #include "sc_text.cuh"
+#include "sc_mtx.cuh"
 #include "bamgpu.cuh"
 
 #include <algorithm>

@@ -5,6 +5,7 @@ One BAM counted by all GPUs of a node:
         -m te_counter_b200.sharded --glb genes_tes.glb --bam in.bam --mode se -o out.tsv
     ... --mode pe -o out.tsv
     ... --mode sc --whitelist 3M-february-2018.txt --maxcells 10000 [--strand] -o out.tsv
+    ... --mode sc --format mtx ... -o out_dir      (matrix.mtx.gz, features.tsv.gz, barcodes.tsv.gz; measureTE.sc_save_mtx)
 
 Every rank builds the same `measureTE` the reference's bin/te_count builds (bin/te_count:77-120) and calls the same
 method; inside, the ranks split the file by byte ranges (shard.py; paired end pairs records by their global index, so
@@ -26,8 +27,12 @@ def main(argv=None):
     ap.add_argument("--whitelist")
     ap.add_argument("--maxcells", type=int, default=10000)
     ap.add_argument("--strand", action="store_true")
+    ap.add_argument("--format", choices=["tsv", "mtx"], default="tsv",
+                    help="single cell: the reference's dense TSV (default) or a 10x-style Matrix Market directory at -o")
     ap.add_argument("-o", "--out", required=True)
     args = ap.parse_args(argv)
+    if args.format == "mtx" and args.mode != "sc":
+        ap.error("--format mtx needs --mode sc")
     import torch
     import torch.distributed as dist
     from . import measureTE
@@ -49,7 +54,9 @@ def main(argv=None):
     if args.mode == "sc":
         res = mte.sc_parse_bamse(args.bam, UMIS=True, whitelistfilename=args.whitelist, strand=args.strand, log=log,
                                  label=os.path.basename(args.out), maxcells=args.maxcells)
-        if rank == 0:
+        if rank == 0 and args.format == "mtx":
+            mte.sc_save_mtx(res, args.out, maxcells=args.maxcells, log=log)
+        elif rank == 0:
             mte.sc_save_result(res, args.out, maxcells=args.maxcells, log=log)
     else:
         mte.load_genome()

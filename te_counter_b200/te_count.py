@@ -26,6 +26,7 @@ import numpy as np
 from . import _lib
 from . import fastbam as _fastbam
 from . import index as _index
+from . import mtx as _mtx
 from . import reads as _reads
 from . import shard as _shard
 
@@ -454,6 +455,39 @@ class measureTE:
                 for barcode in barcodes_to_do:
                     counts = [str(result[f].get(barcode, 0)) for f in result]
                     oh.write('{}\n'.format('\t'.join([barcode] + counts)))
+
+    def sc_save_mtx(self, result, out_dir, maxcells, log=None, threads=None):
+        '''Extension (not in the reference): the matrix of sc_save_result -- the same cells, in the same order -- as a
+        10x-style Matrix Market directory (matrix.mtx.gz, features.tsv.gz, barcodes.tsv.gz; te_counter_b200/mtx.py)
+        that scanpy.read_10x_mtx and Seurat's Read10X read.  `threads`: gzip threads (default: the usable cores).'''
+        if not isinstance(result, ScResult):
+            raise TypeError('sc_save_mtx takes the ScResult of sc_parse_bamse, not %s' % type(result).__name__)
+        assert out_dir, 'You must specify a directory'
+        assert maxcells, 'You must specify maxcells'
+        threads = threads or _mtx.default_threads()
+
+        log.info('Saving the sparse matrix to "{0}"'.format(out_dir))
+        log.info('Found {0:,} barcodes'.format(len(self.barcodes)))
+        eng = self._engine_obj
+        sel = eng.sc_select(maxcells, len(self._sc_hit[0]))   # sc_save_result's rows: count descending, ties by ascending id
+        barcodes_to_do = [result._id_to_barcode[c] for c in sel.tolist()]
+        if len(self.barcodes) > maxcells:
+            log.info(f'Keeping the best {maxcells:,} barcodes')
+        elif maxcells > len(self.barcodes):
+            log.warning('Asked for {0:,} maxcells, but only {1:,} barcodes found'.format(maxcells, len(self.barcodes)))
+
+        os.makedirs(out_dir, exist_ok=True)
+        path = os.path.join(out_dir, 'matrix.mtx.gz')
+        if hasattr(eng, 'sc_matrix_mtx') and getattr(self, '_sc_device_matrix', True):
+            # the text is formatted on the device (libtecount tec_sc_matrix_mtx) and streamed into the compressors
+            _, n_bytes = eng.sc_matrix_mtx(sel)
+            _mtx.write_gzip(path, lambda fh: eng.sc_matrix_write(fh, n_bytes, chunk=_mtx.PIECE), threads)
+        else:
+            text = _mtx.mtx_text(len(result), result.ensg, result.cell, result.count, sel)
+            _mtx.write_gzip(path, lambda fh: fh.write(text), threads)
+        _mtx.write_gzip(os.path.join(out_dir, 'features.tsv.gz'), lambda fh: fh.write(_mtx.features_text(result.keys())), threads)
+        _mtx.write_gzip(os.path.join(out_dir, 'barcodes.tsv.gz'), lambda fh: fh.write(_mtx.barcodes_text(barcodes_to_do)), threads)
+        log.info('Saved {0}'.format(path))
 
 
 def _write_dense_rows(oh, result, barcodes_to_do):
