@@ -83,6 +83,8 @@ typedef enum tec_status {
 #define TEC_BS_QCFAIL 4         /* "Reads are QC fails" */
 #define TEC_BS_CRASH_ENHANCER 5 /* units at which the reference raises NameError (te_count.py:147) */
 #define TEC_BS_CRASH_NAME 6     /* units at which the reference dies in sys.quit (te_count.py:94) */
+#define TEC_BS_NO_MATE 7        /* pairing by read name: records excluded from pairing plus records left without a
+                                   mate (0 in the other modes) */
 
 /* single-cell statistics block, int64[TEC_SC_NSTATS]  (te_count.py:696-705) */
 #define TEC_SC_NSTATS 16
@@ -167,6 +169,26 @@ int tec_index_upload(tec_ctx* ctx, int32_t n_chrom, const int64_t* chrom_off,
  * finish: counts[n_ensg] and stats[TEC_BULK_NSTATS] to host (either may be NULL).
  */
 int tec_bulk_begin(tec_ctx* ctx, int paired, int qual);
+/* Paired end by read name: tec_bulk_begin(ctx, 2, qual).  For files whose mates are not adjacent (coordinate-sorted
+ * BAMs).  The rule:
+ *   - a record takes part when it is primary and carries exactly one mate flag: 0x1 set, 0x100 and 0x800 clear, exactly
+ *     one of 0x40 (read1) / 0x80 (read2).  Every other record is excluded: neither paired nor counted;
+ *   - records are grouped by their exact QNAME bytes (through a 128-bit key of two independent 64-bit hashes,
+ *     bgzf_dev.h name_key).  Within a name, the k-th read1 in input order pairs with the k-th read2 in input order;
+ *   - each pair is counted as a pair of paired = 1 whose record 2i is that read1 and 2i+1 that read2 (filters on both
+ *     mates, read1's MAPQ and chromosome, both starts).  Mates have identical names, so the name check never fires.
+ * Records arrive through tec_bulk_push_named or tec_bam_count(b, 3, ...) only; the other pushes, tec_bam_count in modes
+ * 0-2 and tec_bam_count_range return TEC_ERR_STATE until the next begin.  tec_bulk_finish and tec_bulk_allreduce end
+ * the input: records still waiting for a mate count as no-mate.  stats[TEC_BS_NO_MATE] = excluded + no-mate records.
+ * tec_get_info: "bulk_name_excluded" (excluded records), "bulk_name_pending_peak" (largest number of records waiting for
+ * their mate after a batch), "bulk_name_ms" (device milliseconds of the pairing stage: sorts and group pass).  A batch
+ * needs fewer than 2^32 - 2^13 records together with the ones still waiting (TEC_ERR_LIMIT); a device allocation that
+ * fails returns TEC_ERR_NOMEM.
+ * tec_bulk_push_named: n records in the usual layout plus samflag[n] (the SAM flag) and the QNAME of record i as bytes
+ * [name_off[i], name_off[i+1]) of `names` (name_off[0] = 0, at most 254 bytes each).  Synchronous. */
+int tec_bulk_push_named(tec_ctx* ctx, int64_t n, const int32_t* start, const int32_t* end, const uint16_t* chrom,
+                        const uint8_t* mapq, const uint8_t* flag, const uint16_t* samflag, const int64_t* name_off,
+                        const char* names);
 int tec_bulk_push(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const int32_t* end,
                   const uint16_t* chrom, const uint8_t* mapq, const uint8_t* flag);
 int tec_bulk_push_dev(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const int32_t* end,
@@ -278,7 +300,8 @@ int tec_sc_matrix_mtx(tec_ctx *ctx, int64_t n_cols, const uint32_t *cells, int64
  * exact check of the record chain).  Usage: tec_bam_open, read the reference names, tec_bam_set_chrom_map
  * (and tec_bam_set_whitelist) exactly as for tbam_*, tec_bulk_begin / tec_sc_begin, tec_bam_count (decodes
  * the whole file into the running count), tec_bulk_finish / tec_sc_finalize, tec_bam_close.
- * mode: 0 single end, 1 paired end, 2 single cell.  On TEC_ERR_UNSUPPORTED start over with libtecbam.
+ * mode: 0 single end, 1 paired end, 2 single cell, 3 paired end by read name (tec_bulk_begin(ctx, 2, qual); whole files
+ * only: tec_bam_count_range refuses it with TEC_ERR_ARG).  On TEC_ERR_UNSUPPORTED start over with libtecbam.
  * Options (tec_set_option): "bam_window_blocks" (BGZF blocks per pass, default 65536: 4.3 GB of inflated bytes
  * in HBM), "bam_lanes" (blocks decoded per warp, default 1).  Limits shared with libtecbam: reference_end comes
  * from the CIGAR field of the record (for alignments of more than 65535 operations that field is the placeholder

@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("TEC_LIB") or os.path.join(_HERE, "libtecount.so")
 
 BULK_NSTATS = 8
-BS_UNITS, BS_ASSIGNED, BS_LOWQ, BS_BADCHROM, BS_QCFAIL, BS_CRASH_ENHANCER, BS_CRASH_NAME = range(7)
+BS_UNITS, BS_ASSIGNED, BS_LOWQ, BS_BADCHROM, BS_QCFAIL, BS_CRASH_ENHANCER, BS_CRASH_NAME, BS_NO_MATE = range(8)
 SC_NSTATS = 16
 (SS_UNITS, SS_INVALID_BARCODE, SS_ALREADY_SEEN, SS_LOWQ, SS_QCFAIL, SS_VALID, SS_ASSIGNED,
  SS_RAW_BARCODES, SS_BUNDLES, SS_CRASH_STRAND, SS_SURVIVORS, SS_SEGMENTS) = range(12)
@@ -47,6 +47,7 @@ SIGNATURES = {
     "tec_bulk_begin": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int]),
     "tec_bulk_push": (ctypes.c_int, [_vp, ctypes.c_int64, _vp, _vp, _vp, _vp, _vp]),
     "tec_bulk_push_dev": (ctypes.c_int, [_vp, ctypes.c_int64, _vp, _vp, _vp, _vp, _vp]),
+    "tec_bulk_push_named": (ctypes.c_int, [_vp, ctypes.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, ctypes.c_char_p]),
     "tec_bulk_finish": (ctypes.c_int, [_vp, _c_i64p, _c_i64p]),
     "tec_bulk_counts_dev": (_vp, [_vp]),
     "tec_sc_begin": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int64]),
@@ -177,7 +178,8 @@ class DeviceBam:
             self._eng._check(self._lib.tec_bam_set_whitelist(self._h, b"".join(enc), off.ctypes.data, len(enc)))
 
     def count(self, mode, qual):
-        """mode 0 single end, 1 paired end, 2 single cell; returns the number of records decoded."""
+        """mode 0 single end, 1 paired end, 2 single cell, 3 paired end by read name (after bulk_begin(..., pairing='name'));
+        returns the number of records decoded."""
         n = ctypes.c_int64(0)
         rc = self._lib.tec_bam_count(self._h, int(mode), int(qual), ctypes.byref(n))
         if rc == 0:
@@ -356,8 +358,22 @@ class Engine:
         self.n_ensg = int(n_ensg)
 
     # -- bulk
-    def bulk_begin(self, paired, qual):
-        self._check(self._lib.tec_bulk_begin(self._h, 1 if paired else 0, int(qual)))
+    def bulk_begin(self, paired, qual, pairing="index"):
+        """pairing='name' (paired end only): mates are paired by read name (include/tecount.h, tec_bulk_begin(ctx, 2, qual));
+        records then go in through bulk_push_named or DeviceBam.count(3, qual)."""
+        if pairing not in ("index", "name"):
+            raise ValueError("pairing must be 'index' or 'name'")
+        mode = (2 if pairing == "name" else 1) if paired else 0
+        self._check(self._lib.tec_bulk_begin(self._h, mode, int(qual)))
+
+    def bulk_push_named(self, n, start, end, chrom, mapq, flag, samflag, name_off, names):
+        """Host records for pairing by read name: the usual columns plus samflag (uint16 SAM flags), name_off (int64[n + 1])
+        and names (the QNAME bytes, concatenated)."""
+        if len(name_off) < int(n) + 1:
+            raise ValueError("name_off needs n + 1 entries")
+        self._check(self._lib.tec_bulk_push_named(self._h, int(n), _ptr(start, np.int32), _ptr(end, np.int32),
+                                                  _ptr(chrom, np.uint16), _ptr(mapq, np.uint8), _ptr(flag, np.uint8),
+                                                  _ptr(samflag, np.uint16), _ptr(name_off, np.int64), bytes(names)))
 
     def bulk_push(self, n, start, end, chrom, mapq, flag):
         self._check(self._lib.tec_bulk_push(self._h, int(n), _ptr(start, np.int32), _ptr(end, np.int32),

@@ -274,7 +274,8 @@ inline int parse_pair(Reader& r, const uint8_t* rec1, int64_t n1, const uint8_t*
  *   int  chain(const BlockDesc*, int n_blocks, int64_t w_end, int32_t n_ref, BlockChain* out) find_start (block 0 starts at 0) + hop per block
  *   int  parse(const BlockDesc*, int n_blocks, const BlockChain* used, const int64_t* base, int64_t n_records, int64_t w_end,
  *              int mode, int qual, const Reader&, int* err, int64_t* err_rec)                 parse_record per record into the columns
- *   int  deliver(int64_t n_records, int mode)                          hand the columns on (tec_*_push_dev / copy out)
+ *   int  deliver(int64_t n_records, int mode)                          hand the columns on (tec_*_push_dev / copy out; MODE_PE_NAME:
+ *                                                                      the rows, keys and roles to the pairing stage, pair_name.cuh)
  * and for paired-end byte ranges (decode_range with MODE_PE):
  *   int  parse_pairs(const BlockChain*, const int64_t* base, int nb, int64_t n_records, int64_t g0, int qual, const Reader&,
  *                    int* err, int64_t* err_rec)                       parse_adjacent_pair per adjacent pair into the two column sets
@@ -463,6 +464,7 @@ template <class Backend>
 int decode_range(Reader& r, Backend& be, int mode, int qual, int window_blocks, uint64_t lo, uint64_t hi, RangeResult* res) {
     if (!r.have_map) return r.fail(E_ARG, "the chromosome map has not been set");
     if (!res || lo > hi) return r.fail(E_ARG, "bad byte range");
+    if (mode == bgzfdev::MODE_PE_NAME) return r.fail(E_ARG, "pairing by read name needs the whole file: no byte ranges");
     if (window_blocks < 1) window_blocks = 1;
     *res = RangeResult();
     const bool paired = mode == bgzfdev::MODE_PE;

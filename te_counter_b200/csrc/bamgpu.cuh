@@ -130,8 +130,8 @@ struct BamGpuBackend {
     int64_t* d_wl_off = nullptr;
     uint8_t* d_wl_bytes = nullptr;
     bool ctx_uploaded = false;
-    bgzfdev::Columns col{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    int64_t col_cap = 0;
+    bgzfdev::Columns col{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    int64_t col_cap = 0, name_col_cap = 0;      // name_col_cap: rows of the MODE_PE_NAME columns (key, role)
     PairSets pairs{};                      // paired-end ranges: the two column sets (separate allocations: aligned for bulk2)
     int64_t* d_pair_off = nullptr;
     int64_t pairs_cap = 0;
@@ -145,7 +145,8 @@ struct BamGpuBackend {
         void* blocks[] = {d_comp, d_ubuf, d_scratch, d_tmp, d_blocks, d_chain, d_base, d_status, d_crc, d_err, d_bulk_ids, d_sc_ids, d_wl_slot,
                           d_wl_off, d_wl_bytes, d_rec_off, col.start, col.end, col.chrom, col.mapq, col.flag, col.cell, col.umi, d_pair_off,
                           pairs.s[0].start, pairs.s[0].end, pairs.s[0].chrom, pairs.s[0].mapq, pairs.s[0].flag,
-                          pairs.s[1].start, pairs.s[1].end, pairs.s[1].chrom, pairs.s[1].mapq, pairs.s[1].flag};
+                          pairs.s[1].start, pairs.s[1].end, pairs.s[1].chrom, pairs.s[1].mapq, pairs.s[1].flag,
+                          col.key_hi, col.key_lo, col.role};
         for (void* p : blocks) ctx->cache.put(p);            // back to the context's block cache: the next file reuses them
     }
     template <class T> cudaError_t dev_alloc(T** out, size_t bytes) {
@@ -354,6 +355,14 @@ struct BamGpuBackend {
             BAM_CK(dev_alloc(&col.umi, cap * 8));
             BAM_CK(dev_alloc(&d_rec_off, cap * 8));
             col_cap = (int64_t)cap;
+        }
+        if (mode == bgzfdev::MODE_PE_NAME && name_col_cap < col_cap) {
+            BAM_CK(cudaStreamSynchronize(ctx->stream));
+            dev_free(col.key_hi); dev_free(col.key_lo); dev_free(col.role);
+            name_col_cap = 0;
+            BAM_CK(dev_alloc(&col.key_hi, (size_t)col_cap * 8)); BAM_CK(dev_alloc(&col.key_lo, (size_t)col_cap * 8));
+            BAM_CK(dev_alloc(&col.role, (size_t)col_cap));
+            name_col_cap = col_cap;
         }
         bgzfdev::ParseCtx pc;
         pc.bulk_ids = d_bulk_ids; pc.sc_ids = d_sc_ids; pc.n_ref = (int32_t)r.refs.size(); pc.n_index = r.n_index; pc.qual = qual;

@@ -474,6 +474,7 @@ struct Rec {
     uint32_t l_name;            // without the NUL
     const uint8_t *name, *aux, *aux_end;
     uint8_t mapq, fbits;
+    uint16_t flag;              // the SAM flag
     bool has_end, ok;
 };
 
@@ -483,6 +484,7 @@ BGZF_HD Rec parse_core(const uint8_t* p, uint32_t n) {      // p behind block_si
     c.pos = (int32_t)ld32(p + 4);
     const uint32_t l_name = p[8], n_cig = ld16(p + 12), flag = ld16(p + 14);
     c.mapq = p[9];
+    c.flag = (uint16_t)flag;
     const int64_t l_seq = (int32_t)ld32(p + 16);
     c.fbits = (uint8_t)(((flag >> 2) & 1) * F_UNMAPPED | ((flag >> 10) & 1) * F_DUP | ((flag >> 9) & 1) * F_QCFAIL | ((flag >> 4) & 1) * F_REVERSE);
     const uint64_t o = 32ull + l_name + 4ull * n_cig;
@@ -616,12 +618,44 @@ BGZF_HD uint32_t wl_find(const WhitelistView& wl, const uint8_t* p, uint32_t n) 
     }
 }
 
+// Paired end by read name (MODE_PE_NAME): the 128-bit key of a QNAME, two independent 64-bit hashes of its bytes
+// (FNV-1a and a multiply-xorshift hash, each through the splitmix64 finalizer).  Mates compare keys, never bytes: for
+// 10^9 distinct names the chance that any two share a key is about n^2 / 2^129 = 1.5e-21.
+BGZF_HD uint64_t mix64(uint64_t h) {
+    h ^= h >> 30;
+    h *= 0xbf58476d1ce4e5b9ull;
+    h ^= h >> 27;
+    h *= 0x94d049bb133111ebull;
+    return h ^ (h >> 31);
+}
+
+BGZF_HD void name_key(const uint8_t* p, uint32_t n, uint64_t& hi, uint64_t& lo) {
+    uint64_t a = 0xcbf29ce484222325ull, b = 0x9e3779b97f4a7c15ull ^ n;
+    for (uint32_t i = 0; i < n; i++) {
+        a = (a ^ p[i]) * 0x100000001b3ull;
+        b = (b + p[i] + 1) * 0xff51afd7ed558ccdull;
+        b ^= b >> 29;
+    }
+    hi = mix64(a ^ ((uint64_t)n << 56));
+    lo = mix64(b);
+}
+
+// which side of a pair a record is on: primary (0x100, 0x800 clear), paired (0x1) and exactly one of 0x40 / 0x80
+enum { ROLE_EXCLUDED = 0, ROLE_READ1 = 1, ROLE_READ2 = 2 };
+BGZF_HD int name_role(uint32_t flag) {
+    if (!(flag & 0x1) || (flag & 0x900)) return ROLE_EXCLUDED;
+    const uint32_t m = flag & 0xC0;
+    return m == 0x40 ? ROLE_READ1 : m == 0x80 ? ROLE_READ2 : ROLE_EXCLUDED;
+}
+
 struct Columns {
     int32_t *start, *end;
     uint16_t* chrom;
     uint8_t *mapq, *flag;
     uint32_t* cell;
     uint64_t* umi;
+    uint64_t *key_hi, *key_lo;  // MODE_PE_NAME: name_key of the QNAME (0 for excluded records)
+    uint8_t* role;              // MODE_PE_NAME: name_role of the SAM flag
 };
 
 struct ParseCtx {
@@ -630,10 +664,12 @@ struct ParseCtx {
     WhitelistView wl;
 };
 
-enum { MODE_SE = 0, MODE_PE = 1, MODE_SC = 2 };
+enum { MODE_SE = 0, MODE_PE = 1, MODE_SC = 2, MODE_PE_NAME = 3 };
 
 // Record at window offset p (complete by construction) into row k.  For MODE_PE the caller passes
-// the FIRST mate and p2 = offset of the second; rows k and k + 1 are written.  Returns E_*.
+// the FIRST mate and p2 = offset of the second; rows k and k + 1 are written.  MODE_PE_NAME writes the
+// one-record row of MODE_SE plus the name key and the role; the pairing stage (pair_name.cuh) makes the
+// pairs.  Returns E_*.
 BGZF_HD int parse_record(const uint8_t* w, int64_t p, int64_t p2, int mode, const ParseCtx& pc, const Columns& o, int64_t k) {
     const Rec c = parse_core(w + p + 4, ld32(w + p));
     if (!c.ok) return E_FORMAT;
@@ -649,6 +685,15 @@ BGZF_HD int parse_record(const uint8_t* w, int64_t p, int64_t p2, int mode, cons
         const bool has_ref2 = c2.ref_id >= 0 && c2.ref_id < pc.n_ref;
         o.start[k + 1] = c2.pos; o.end[k + 1] = c2.end; o.chrom[k + 1] = has_ref2 ? pc.bulk_ids[c2.ref_id] : (uint16_t)CHROM_INVALID;
         o.mapq[k + 1] = c2.mapq; o.flag[k + 1] = c2.fbits;
+        return E_NONE;
+    }
+    if (mode == MODE_PE_NAME) {
+        o.start[k] = c.pos; o.end[k] = c.end; o.chrom[k] = has_ref ? pc.bulk_ids[c.ref_id] : (uint16_t)CHROM_INVALID;
+        o.mapq[k] = c.mapq; o.flag[k] = c.fbits;
+        const int role = name_role(c.flag);
+        uint64_t hi = 0, lo = 0;
+        if (role != ROLE_EXCLUDED) name_key(c.name, c.l_name, hi, lo);
+        o.key_hi[k] = hi; o.key_lo[k] = lo; o.role[k] = (uint8_t)role;
         return E_NONE;
     }
     if (mode == MODE_SE) {

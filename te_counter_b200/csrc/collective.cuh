@@ -133,5 +133,6 @@ extern "C" int tec_bulk_allreduce(tec_ctx* ctx) {
     if (ctx->bank_pending) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_allreduce: a paired-end range count waits for tec_bulk_keep_bank");
     if (!ctx->comm) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_allreduce: tec_comm_init not called");
     TEC_CUDA(cudaSetDevice(ctx->device));
+    if (int rc = name_flush(ctx)) return rc;
     return comm_allreduce(ctx, ctx->d_counts, (int64_t)ctx->idx.n_ensg + TEC_BULK_NSTATS, 1, 0);
 }

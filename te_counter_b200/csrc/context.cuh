@@ -84,6 +84,9 @@ struct StageSlot {
 };
 
 struct ScState;      // sc.cuh
+struct NameState;    // pair_name.cuh
+struct tec_ctx;
+static int name_flush(tec_ctx* ctx);     // pair_name.cuh: the rows still pending count as no-mate
 
 // Size-keyed cache of device blocks: the single-cell finalize asks for the same sequence of
 // temporaries on every call, and cudaMalloc / cudaFree (a device-wide synchronisation each) would
@@ -153,6 +156,8 @@ struct tec_ctx {
     u64* d_counts = nullptr;              // n_ensg counters (slot order) + TEC_BULK_NSTATS statistics
     u64* d_bank1 = nullptr;               // paired-end byte range: the counters of the pairs of odd range-local index (same layout)
     bool bank_pending = false;            // a paired-end range count waits for tec_bulk_keep_bank
+    bool name_pairing = false;            // tec_bulk_begin(ctx, 2, qual): mates paired by read name (pair_name.cuh)
+    NameState* name = nullptr;
     u32* d_slow_list = nullptr;           // [0] = count, then unit indices flagged for bulk_slow_kernel
     int64_t slow_cap = 0;                 // words
     void* d_ring = nullptr;               // per-warp second deferral ring of the fast bulk kernel (QEnt)
@@ -207,6 +212,7 @@ struct tec_ctx {
     void free_stage();
     void free_index();
     void free_sc();
+    void free_name();
     void free_bam() {
         for (int i = 0; i < 2; i++) {
             if (bam_pinned[i]) cudaFreeHost(bam_pinned[i]);
@@ -219,7 +225,7 @@ struct tec_ctx {
         if (bam_stream2) cudaStreamDestroy(bam_stream2);
         bam_stream2 = nullptr;
     }
-    void free_all() { free_stage(); free_index(); free_sc(); free_bam(); cache.trim(); }
+    void free_all() { free_stage(); free_index(); free_sc(); free_name(); free_bam(); cache.trim(); }
 };
 
 inline void tec_ctx::free_stage() {

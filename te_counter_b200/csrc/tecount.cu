@@ -9,6 +9,7 @@
 #include "sc_text.cuh"
 #include "sc_mtx.cuh"
 #include "bamgpu.cuh"
+#include "pair_name.cuh"
 
 #include <algorithm>
 #include <cstdio>
@@ -331,7 +332,11 @@ extern "C" int tec_bulk_begin(tec_ctx* ctx, int paired, int qual) {
     if (!ctx->has_index) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_begin: no index uploaded");
     TEC_CUDA(cudaSetDevice(ctx->device));
     ctx->paired = paired ? 1 : 0;
+    ctx->name_pairing = paired == 2;
     ctx->qual = qual;
+    ctx->bulk_active = false;
+    if (ctx->name_pairing)
+        if (int rc = name_begin(ctx)) return rc;
     TEC_CUDA(cudaMemsetAsync(ctx->d_counts, 0, ((size_t)ctx->idx.n_ensg + TEC_BULK_NSTATS) * 8, ctx->stream));
     ctx->bulk_active = true;
     ctx->bank_pending = false;
@@ -342,6 +347,13 @@ extern "C" int tec_bulk_begin(tec_ctx* ctx, int paired, int qual) {
 static int bulk_ready(tec_ctx* ctx, const char* what) {
     if (!ctx->bulk_active) TEC_FAIL(TEC_ERR_STATE, std::string(what) + ": tec_bulk_begin not called");
     if (ctx->bank_pending) TEC_FAIL(TEC_ERR_STATE, std::string(what) + ": a paired-end range count waits for tec_bulk_keep_bank");
+    return TEC_OK;
+}
+
+// ... and for the pushes of records that are already pairs: not in the run of name pairing
+static int bulk_ready_pairs(tec_ctx* ctx, const char* what) {
+    if (int rc = bulk_ready(ctx, what)) return rc;
+    if (ctx->name_pairing) TEC_FAIL(TEC_ERR_STATE, std::string(what) + ": the run pairs mates by read name (tec_bulk_push_named, tec_bam_count mode 3)");
     return TEC_OK;
 }
 
@@ -574,7 +586,7 @@ static int bulk_push_dev(tec_ctx* ctx, int64_t n_rec, const int32_t* start, cons
 extern "C" int tec_bulk_push_dev(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const int32_t* end,
                                  const uint16_t* chrom, const uint8_t* mapq, const uint8_t* flag) {
     if (!ctx) return TEC_ERR_ARG;
-    if (int rc = bulk_ready(ctx, "tec_bulk_push_dev")) return rc;
+    if (int rc = bulk_ready_pairs(ctx, "tec_bulk_push_dev")) return rc;
     return bulk_push_dev(ctx, n_rec, start, end, chrom, mapq, flag);
 }
 
@@ -583,7 +595,7 @@ extern "C" int tec_bulk_push_dev(tec_ctx* ctx, int64_t n_rec, const int32_t* sta
 extern "C" int tec_bulk_push(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const int32_t* end,
                              const uint16_t* chrom, const uint8_t* mapq, const uint8_t* flag) {
     if (!ctx) return TEC_ERR_ARG;
-    if (int rc = bulk_ready(ctx, "tec_bulk_push")) return rc;
+    if (int rc = bulk_ready_pairs(ctx, "tec_bulk_push")) return rc;
     if (n_rec < 0 || (ctx->paired && (n_rec & 1))) TEC_FAIL(TEC_ERR_ARG, "tec_bulk_push: record count must be even in paired mode");
     if (n_rec == 0) return TEC_OK;
     if (!start || !end || !chrom || !mapq || !flag) TEC_FAIL(TEC_ERR_ARG, "tec_bulk_push: null array");
@@ -618,10 +630,29 @@ extern "C" int tec_bulk_push(tec_ctx* ctx, int64_t n_rec, const int32_t* start, 
     return TEC_OK;
 }
 
+extern "C" int tec_bulk_push_named(tec_ctx* ctx, int64_t n, const int32_t* start, const int32_t* end, const uint16_t* chrom,
+                                   const uint8_t* mapq, const uint8_t* flag, const uint16_t* samflag, const int64_t* name_off,
+                                   const char* names) {
+    if (!ctx) return TEC_ERR_ARG;
+    if (int rc = bulk_ready(ctx, "tec_bulk_push_named")) return rc;
+    if (!ctx->name_pairing) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_push_named: tec_bulk_begin was not called with paired = 2");
+    if (n < 0) TEC_FAIL(TEC_ERR_ARG, "tec_bulk_push_named: negative record count");
+    if (n == 0) return TEC_OK;
+    if (!start || !end || !chrom || !mapq || !flag || !samflag || !name_off || (name_off[n] > 0 && !names))
+        TEC_FAIL(TEC_ERR_ARG, "tec_bulk_push_named: null array");
+    if (name_off[0] != 0) TEC_FAIL(TEC_ERR_ARG, "tec_bulk_push_named: name_off[0] must be 0");
+    for (int64_t i = 0; i < n; ++i)
+        if (name_off[i + 1] < name_off[i] || name_off[i + 1] - name_off[i] > 254)
+            TEC_FAIL(TEC_ERR_ARG, "tec_bulk_push_named: name_off must ascend by at most 254 bytes per name");
+    TEC_CUDA(cudaSetDevice(ctx->device));
+    return name_push_host(ctx, n, start, end, chrom, mapq, flag, samflag, name_off, names);
+}
+
 extern "C" int tec_bulk_finish(tec_ctx* ctx, int64_t* counts, int64_t* stats) {
     if (!ctx) return TEC_ERR_ARG;
     if (int rc = bulk_ready(ctx, "tec_bulk_finish")) return rc;
     TEC_CUDA(cudaSetDevice(ctx->device));
+    if (int rc = name_flush(ctx)) return rc;
     const size_t ne = (size_t)ctx->idx.n_ensg;
     std::vector<int64_t> tmp(ne + TEC_BULK_NSTATS);
     TEC_CUDA(cudaMemcpyAsync(tmp.data(), ctx->d_counts, (ne + TEC_BULK_NSTATS) * 8, cudaMemcpyDeviceToHost, ctx->stream));
@@ -701,6 +732,9 @@ extern "C" int64_t tec_get_info(tec_ctx* ctx, const char* key) {
     if (k == "sc_stab_bytes") return (int64_t)ctx->idx.sc_stab_bytes;
     if (k == "n_sm") return ctx->n_sm;
     if (k == "sc_last_sort") return ctx->sc_last_sort;
+    if (k == "bulk_name_excluded") return ctx->name_pairing && ctx->name ? ctx->name->excluded : 0;
+    if (k == "bulk_name_pending_peak") return ctx->name_pairing && ctx->name ? ctx->name->peak : 0;
+    if (k == "bulk_name_ms") return ctx->name_pairing && ctx->name ? (int64_t)(ctx->name->ms + 0.5) : 0;
     if (k == "sc_last_sort_passes") return ctx->sc_last_sort_passes;
     if (k == "n_features") return ctx->idx.n_feat;
     if (k == "last_slow_units") {          // units the last fast-kernel launch handed to the exact kernel
@@ -719,6 +753,11 @@ extern "C" int64_t tec_get_info(tec_ctx* ctx, const char* key) {
 // ------------------------------------------------------------------------------------------------
 // BAM file -> counting path on the device (bamgpu.cuh)
 int BamGpuBackend::deliver(int64_t n, int mode) {
+    if (mode == bgzfdev::MODE_PE_NAME) {
+        const int rc = name_push_dev(ctx, n, col);
+        nomem = rc == TEC_ERR_NOMEM;
+        return rc ? 1 : 0;
+    }
     const int rc = mode == bgzfdev::MODE_SC
                        ? tec_sc_push_dev(ctx, n, col.start, col.end, col.chrom, col.mapq, col.flag, col.cell, col.umi)
                        : tec_bulk_push_dev(ctx, n, col.start, col.end, col.chrom, col.mapq, col.flag);
@@ -796,10 +835,11 @@ extern "C" int tec_bam_count(tec_bam* b, int mode, int qual, int64_t* n_records)
     if (!b) return TEC_ERR_ARG;
     tec_ctx* ctx = b->ctx;
     if (n_records) *n_records = 0;
-    if (mode < 0 || mode > 2) TEC_FAIL(TEC_ERR_ARG, "tec_bam_count: mode must be 0 (single end), 1 (paired end) or 2 (single cell)");
+    if (mode < 0 || mode > 3)
+        TEC_FAIL(TEC_ERR_ARG, "tec_bam_count: mode must be 0 (single end), 1 (paired end), 2 (single cell) or 3 (paired end by read name)");
     if (mode == bgzfdev::MODE_SC) {
         if (!ctx->sc || !ctx->sc->active) TEC_FAIL(TEC_ERR_STATE, "tec_bam_count: tec_sc_begin not called");
-    } else if (!ctx->bulk_active || (ctx->paired ? 1 : 0) != mode) {
+    } else if (!ctx->bulk_active || (ctx->name_pairing ? 3 : ctx->paired ? 1 : 0) != mode) {
         TEC_FAIL(TEC_ERR_STATE, "tec_bam_count: tec_bulk_begin not called for this mode");
     } else if (int st = bulk_ready(ctx, "tec_bam_count")) {
         return st;
@@ -820,7 +860,7 @@ extern "C" int tec_bam_count_range(tec_bam* b, int mode, int qual, int64_t byte_
     if (byte_lo < 0 || byte_hi < byte_lo) TEC_FAIL(TEC_ERR_ARG, "tec_bam_count_range: bad byte range");
     if (mode == bgzfdev::MODE_SC) {
         if (!ctx->sc || !ctx->sc->active) TEC_FAIL(TEC_ERR_STATE, "tec_bam_count_range: tec_sc_begin not called");
-    } else if (!ctx->bulk_active || (ctx->paired ? 1 : 0) != mode) {
+    } else if (!ctx->bulk_active || (ctx->paired ? 1 : 0) != mode || ctx->name_pairing) {
         TEC_FAIL(TEC_ERR_STATE, "tec_bam_count_range: tec_bulk_begin not called for this mode");
     } else if (int st = bulk_ready(ctx, "tec_bam_count_range")) {
         return st;

@@ -121,9 +121,10 @@ def _flagbits(read):
 
 
 class Batch:
-    """Preallocated SoA buffers (pinned when the library hands out the memory)."""
+    """Preallocated SoA buffers (pinned when the library hands out the memory).  named: pairing by read name also
+    carries each record's SAM flag and QNAME (fill_bulk_named)."""
 
-    def __init__(self, capacity, sc=False, alloc=None):
+    def __init__(self, capacity, sc=False, alloc=None, named=False):
         alloc = alloc or (lambda n, dt: np.empty(n, dtype=dt))
         self.capacity = capacity
         self.start = alloc(capacity, np.int32)
@@ -133,6 +134,9 @@ class Batch:
         self.flag = alloc(capacity, np.uint8)
         self.cell = alloc(capacity, np.uint32) if sc else None
         self.umi = alloc(capacity, np.uint64) if sc else None
+        self.samflag = alloc(capacity, np.uint16) if named else None
+        self.name_off = np.zeros(capacity + 1, dtype=np.int64) if named else None
+        self.names = b""
         self.n = 0
 
 
@@ -196,6 +200,38 @@ def fill_bulk(batch, sam, chrom_map, paired, qual):
             mapq[n] = int(r1.mapping_quality)
             flag[n] = f1
             n += 1
+    batch.n = n
+    return more
+
+
+def fill_bulk_named(batch, sam, chrom_map):
+    """Pairing by read name (libtecount tec_bulk_push_named): one row per record in file order, as for single end,
+    plus its SAM flag and its QNAME bytes (batch.names, record i at [name_off[i], name_off[i + 1])).  Which records
+    pair is decided on the device.  Returns False when the iterator is exhausted."""
+    start, end, chrom, mapq, flag, samflag = batch.start, batch.end, batch.chrom, batch.mapq, batch.flag, batch.samflag
+    names = []
+    n = 0
+    more = True
+    bulk_id = chrom_map.bulk_id
+    while n < batch.capacity:
+        try:
+            r = next(sam)
+        except StopIteration:
+            more = False
+            break
+        s, e = r.reference_start, r.reference_end
+        start[n] = s if s is not None else -1
+        end[n] = e if e is not None else -1
+        chrom[n] = bulk_id(r.reference_name)
+        mapq[n] = int(r.mapping_quality)
+        flag[n] = _flagbits(r)
+        samflag[n] = int(r.flag)
+        names.append(r.query_name.encode())
+        n += 1
+    batch.name_off[0] = 0
+    if n:
+        np.cumsum([len(x) for x in names], out=batch.name_off[1:n + 1])
+    batch.names = b"".join(names)
     batch.n = n
     return more
 

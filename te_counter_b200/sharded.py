@@ -4,6 +4,7 @@ One BAM counted by all GPUs of a node:
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29500 \\
         -m te_counter_b200.sharded --glb genes_tes.glb --bam in.bam --mode se -o out.tsv
     ... --mode pe -o out.tsv
+    ... --mode pe --pairing name -o out.tsv      (coordinate-sorted BAM: mates paired by read name, decoded by rank 0)
     ... --mode sc --whitelist 3M-february-2018.txt --maxcells 10000 [--strand] -o out.tsv
     ... --mode sc --format mtx ... -o out_dir      (matrix.mtx.gz, features.tsv.gz, barcodes.tsv.gz; measureTE.sc_save_mtx)
 
@@ -29,10 +30,14 @@ def main(argv=None):
     ap.add_argument("--strand", action="store_true")
     ap.add_argument("--format", choices=["tsv", "mtx"], default="tsv",
                     help="single cell: the reference's dense TSV (default) or a 10x-style Matrix Market directory at -o")
+    ap.add_argument("--pairing", choices=["index", "name"], default="index",
+                    help="paired end: record 2i with 2i+1 as the reference (default), or mates by read name (measureTE.parse_bampe)")
     ap.add_argument("-o", "--out", required=True)
     args = ap.parse_args(argv)
     if args.format == "mtx" and args.mode != "sc":
         ap.error("--format mtx needs --mode sc")
+    if args.pairing == "name" and args.mode != "pe":
+        ap.error("--pairing name needs --mode pe")
     import torch
     import torch.distributed as dist
     from . import measureTE
@@ -60,7 +65,10 @@ def main(argv=None):
             mte.sc_save_result(res, args.out, maxcells=args.maxcells, log=log)
     else:
         mte.load_genome()
-        res = (mte.parse_bampe if args.mode == "pe" else mte.parse_bamse)(args.bam, log=log)
+        if args.mode == "pe":
+            res = mte.parse_bampe(args.bam, log=log, pairing=args.pairing)
+        else:
+            res = mte.parse_bamse(args.bam, log=log)
         if rank == 0:
             mte.save_result_bulk(res, args.out, log=log)
     if world > 1:

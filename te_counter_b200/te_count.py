@@ -35,9 +35,10 @@ SC_BUNDLE_KEYS = 10000000        # te_count.py:377  `len(umis) >= 1e7`
 SC_CELL_PAD = 1000               # te_count.py:502  `maxcells+1000`
 
 
-def _open_alignment(filename, tags_optional=False):
+def _open_alignment(filename, tags_optional=False, by_name=False):
     """Host readers.  tags_optional (the --noumi extension): only the readers with pysam's interface, whose
-    records are packed by reads.fill_sc, can leave the UMI tags unread.
+    records are packed by reads.fill_sc, can leave the UMI tags unread.  by_name (parse_bampe(pairing='name')): only
+    they hand out QNAMEs and SAM flags (reads.fill_bulk_named); libtecbam does not.
       TEC_BAM_DECODER = auto (default) | gpu | native | pysam | python.  `auto` / `gpu`:
     the callers first try the device decoder (tec_bam_*) and come here only for files it refuses;
     then block-compressed BAM goes through libtecbam (threads inflate and parse into the pinned
@@ -49,7 +50,7 @@ def _open_alignment(filename, tags_optional=False):
         raise ValueError('TEC_BAM_DECODER must be auto, gpu, native, pysam or python')
     if mode == 'gpu':
         mode = 'auto'
-    if not tags_optional and (mode == 'native' or (mode == 'auto' and _fastbam.available())):
+    if not (tags_optional or by_name) and (mode == 'native' or (mode == 'auto' and _fastbam.available())):
         try:
             return _fastbam.NativeBam(filename)
         except (_fastbam.NotBgzf, OSError):             # SAM text, plain gzip, not a regular file: next reader
@@ -170,22 +171,27 @@ class measureTE:
         self.genelist_glb_filename = genelist_glb_filename
 
     # ---------------------------------------------------------------- bulk
-    def _parse_bulk(self, filename, strand, log, paired):
+    def _parse_bulk(self, filename, strand, log, paired, pairing='index'):
         assert filename, 'You must specify a filename'
+        if pairing not in ('index', 'name'):
+            raise ValueError("pairing must be 'index' or 'name', not %r" % (pairing,))
         if strand and not self.extensions:
             raise NotImplementedError()                       # te_count.py:58-59 / :183-184
         qual = self._qual()
         eng = self._engine()
         eng.set_option('bulk_strand', 1 if strand else 0)     # extension: strand-aware candidates (exact-search kernel)
         try:
-            return self._parse_bulk_run(eng, filename, log, paired, qual)
+            return self._parse_bulk_run(eng, filename, log, paired, qual, pairing == 'name')
         finally:
             eng.set_option('bulk_strand', 0)
 
-    def _parse_bulk_run(self, eng, filename, log, paired, qual):
+    def _parse_bulk_run(self, eng, filename, log, paired, qual, by_name=False):
         cm = _reads.ChromMap(self.genome.chrom_keys)
         label = 'reads' if paired else 'SE reads'
         more, done, next_log = True, 0, 1000000
+        # pairing by read name: pairs are only known once the pairing stage has seen their mates, so the progress lines
+        # are written from the final pair count; a sharded run decodes the whole file on rank 0
+        begin = (lambda: eng.bulk_begin(paired, qual, pairing='name')) if by_name else (lambda: eng.bulk_begin(paired, qual))
         # One file, several ranks (torch.distributed job, one process per GPU; shard.py): every rank decodes a byte range
         # on its GPU and the counters are summed; paired end keeps the counter bank of the rank's record parity and
         # counts the pair across its front border.  Files whose ranges the decoders cannot tile are decoded by rank 0
@@ -194,7 +200,7 @@ class measureTE:
         in_library = _shard.join_collectives(eng) if world > 1 else False
         if world > 1:
             sharded = None
-            if _device_decoder_wanted(eng):
+            if _device_decoder_wanted(eng) and not by_name:
                 def open_and_bind():
                     dev = eng.bam_open(filename)
                     dev.bind(cm)
@@ -211,16 +217,16 @@ class measureTE:
                     done //= 2
                 log.info('{:,} of them decoded by this rank ({} of {})'.format(sharded[0], rank, world))
             elif rank != 0:
-                eng.bulk_begin(paired, qual)                  # nothing to decode here: rank 0 reads the whole file
+                begin()                                       # nothing to decode here: rank 0 reads the whole file
                 more = False
         if more and _device_decoder_wanted(eng):
             try:                                              # BGZF inflate, record split and packing on the device
                 dev = eng.bam_open(filename)
                 try:
                     dev.bind(cm)
-                    eng.bulk_begin(paired, qual)
-                    done = dev.count(1 if paired else 0, qual)
-                    done = done // 2 if paired else done
+                    begin()
+                    done = dev.count(3 if by_name else 1 if paired else 0, qual)
+                    done = 0 if by_name else done // 2 if paired else done
                     more = False
                     self._bam_info = dev.info()
                 finally:
@@ -238,12 +244,16 @@ class measureTE:
         sam = batch = None
         if more:
             done, next_log = 0, 1000000
-            sam = _open_alignment(filename)
+            sam = _open_alignment(filename, by_name=by_name)
             native = isinstance(sam, _fastbam.NativeBam)
             if native:
                 sam.bind(cm)
-            batch = _reads.Batch(BATCH_RECORDS, alloc=eng.pinned)
-            eng.bulk_begin(paired, qual)
+            batch = _reads.Batch(BATCH_RECORDS, alloc=eng.pinned, named=by_name)
+            begin()
+        while more and by_name:
+            more = _reads.fill_bulk_named(batch, sam, cm)
+            eng.bulk_push_named(batch.n, batch.start, batch.end, batch.chrom, batch.mapq, batch.flag, batch.samflag,
+                                batch.name_off, batch.names)
         while more:
             more = sam.fill_bulk(batch, paired, qual) if native else _reads.fill_bulk(batch, sam, cm, paired, qual)
             eng.bulk_push(batch.n, batch.start, batch.end, batch.chrom, batch.mapq, batch.flag)
@@ -259,6 +269,10 @@ class measureTE:
         if world > 1 and not in_library:
             from . import dist as _tdist
             counts, st = _tdist.allreduce_counts_host(counts, st)
+        if by_name:
+            while int(st[_lib.BS_UNITS]) >= next_log:
+                log.info('Processed {:,} {}'.format(next_log, label))
+                next_log += 1000000
         if st[_lib.BS_CRASH_NAME]:
             log.error('Unmatched pair!')
             raise AttributeError("module 'sys' has no attribute 'quit'")      # te_count.py:94
@@ -272,12 +286,21 @@ class measureTE:
         log.info('{:,} Read quality is too low (<{})'.format(int(st[_lib.BS_LOWQ]), self.quality_threshold))
         log.info('{:,} Reads mapped to an invalid chromosome'.format(int(st[_lib.BS_BADCHROM])))
         log.info('{:,} Reads are QC fails'.format(int(st[_lib.BS_QCFAIL])))
+        if by_name:
+            excluded = eng.get_info('bulk_name_excluded')
+            log.info('{:,} records were not paired by name: {:,} not primary or without exactly one mate flag, {:,} without '
+                     'a mate'.format(int(st[_lib.BS_NO_MATE]), excluded, int(st[_lib.BS_NO_MATE]) - excluded))
         self.total_reads = idx
         return dict(zip(self.all_feature_names, counts.tolist()))
 
-    def parse_bampe(self, filename, strand=False, log=None):
-        '''Load in a BAMPE file (reference te_count.py:42-165)'''
-        return self._parse_bulk(filename, strand, log, True)
+    def parse_bampe(self, filename, strand=False, log=None, pairing='index'):
+        '''Load in a BAMPE file (reference te_count.py:42-165).
+
+        pairing (extension): 'index' (default) pairs records as the reference does, record 2i with record 2i+1, which is
+        only right for a name-collated file.  'name' pairs the k-th read1 of a read name with its k-th read2 wherever
+        they lie (coordinate-sorted BAMs: STAR SortedByCoordinate, samtools sort); only primary records with exactly one
+        of the flags 0x40 / 0x80 (and 0x1) take part.  The result equals the reference's on the name-collated pairs.'''
+        return self._parse_bulk(filename, strand, log, True, pairing)
 
     def parse_bamse(self, filename, strand=False, log=None):
         '''Load in a BAMSE file (reference te_count.py:167-277)'''

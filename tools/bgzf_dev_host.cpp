@@ -15,13 +15,15 @@ struct HostBackend {
     std::vector<uint16_t> c_chrom;
     std::vector<uint8_t> c_mapq, c_flag;
     std::vector<uint32_t> c_cell;
-    std::vector<uint64_t> c_umi;
+    std::vector<uint64_t> c_umi, c_key_hi, c_key_lo;
+    std::vector<uint8_t> c_role;
     // everything delivered so far
     std::vector<int32_t> o_start, o_end;
     std::vector<uint16_t> o_chrom;
     std::vector<uint8_t> o_mapq, o_flag;
     std::vector<uint32_t> o_cell;
-    std::vector<uint64_t> o_umi;
+    std::vector<uint64_t> o_umi, o_key_hi, o_key_lo;      // MODE_PE_NAME: name keys and roles
+    std::vector<uint8_t> o_role;
     // paired-end ranges: the two column sets of the window, and everything delivered into each
     struct Set {
         std::vector<int32_t> start, end;
@@ -88,8 +90,9 @@ struct HostBackend {
     int parse(const bamorch::BlockDesc* bl, int nb, const bamorch::BlockChain* ch, const int64_t* base, int64_t n, int64_t, int mode, int qual,
               const bamorch::Reader& r, int* err, int64_t* err_rec) {
         c_start.resize((size_t)n); c_end.resize((size_t)n); c_chrom.resize((size_t)n); c_mapq.resize((size_t)n); c_flag.resize((size_t)n);
-        c_cell.resize((size_t)n); c_umi.resize((size_t)n);
-        bgzfdev::Columns o{c_start.data(), c_end.data(), c_chrom.data(), c_mapq.data(), c_flag.data(), c_cell.data(), c_umi.data()};
+        c_cell.resize((size_t)n); c_umi.resize((size_t)n); c_key_hi.resize((size_t)n); c_key_lo.resize((size_t)n); c_role.resize((size_t)n);
+        bgzfdev::Columns o{c_start.data(), c_end.data(), c_chrom.data(), c_mapq.data(), c_flag.data(), c_cell.data(), c_umi.data(),
+                           c_key_hi.data(), c_key_lo.data(), c_role.data()};
         bgzfdev::ParseCtx pc;
         pc.bulk_ids = r.bulk_ids.data(); pc.sc_ids = r.sc_ids.data(); pc.n_ref = (int32_t)r.refs.size(); pc.n_index = r.n_index; pc.qual = qual;
         pc.wl.slot = r.wl_slot.data(); pc.wl.off = r.wl_off.data(); pc.wl.bytes = (const uint8_t*)r.wl_bytes.data();
@@ -168,6 +171,11 @@ struct HostBackend {
         if (mode == bgzfdev::MODE_SC) {
             o_cell.insert(o_cell.end(), c_cell.begin(), c_cell.begin() + n);
             o_umi.insert(o_umi.end(), c_umi.begin(), c_umi.begin() + n);
+        }
+        if (mode == bgzfdev::MODE_PE_NAME) {        // the device hands these to the pairing stage (pair_name.cuh)
+            o_key_hi.insert(o_key_hi.end(), c_key_hi.begin(), c_key_hi.begin() + n);
+            o_key_lo.insert(o_key_lo.end(), c_key_lo.begin(), c_key_lo.begin() + n);
+            o_role.insert(o_role.end(), c_role.begin(), c_role.begin() + n);
         }
         return 0;
     }
@@ -280,6 +288,20 @@ uint32_t bgzfdev_crc32_lanes(const void* p, int64_t n) {
 
 // the whitelist hash of the decoder (bgzf_dev.h), for holding its numpy restatement against it
 uint64_t bgzfdev_wl_hash(const void* p, uint32_t n) { return bgzfdev::wl_hash((const uint8_t*)p, n); }
+
+// the read-name key and the pairing role of bgzf_dev.h, likewise; key[0] = high word, key[1] = low word
+void bgzfdev_name_key(const void* p, uint32_t n, uint64_t* key) { bgzfdev::name_key((const uint8_t*)p, n, key[0], key[1]); }
+int bgzfdev_name_role(uint32_t flag) { return bgzfdev::name_role(flag); }
+
+// the name keys and roles delivered so far in MODE_PE_NAME (as many as bgzfdev_fetch's rows)
+void bgzfdev_fetch_named(void* h, uint64_t* key_hi, uint64_t* key_lo, uint8_t* role) {
+    HostBackend& b = ((Session*)h)->be;
+    const size_t n = b.o_key_hi.size();
+    if (!n) return;
+    memcpy(key_hi, b.o_key_hi.data(), n * 8);
+    memcpy(key_lo, b.o_key_lo.data(), n * 8);
+    memcpy(role, b.o_role.data(), n);
+}
 
 // the block inflate alone, for holding it against zlib
 int bgzfdev_inflate_raw(const void* in, int64_t n_in, void* out, int64_t n_out) {
