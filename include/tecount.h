@@ -177,8 +177,8 @@ int tec_bulk_begin(tec_ctx* ctx, int paired, int qual);
  *     bgzf_dev.h name_key).  Within a name, the k-th read1 in input order pairs with the k-th read2 in input order;
  *   - each pair is counted as a pair of paired = 1 whose record 2i is that read1 and 2i+1 that read2 (filters on both
  *     mates, read1's MAPQ and chromosome, both starts).  Mates have identical names, so the name check never fires.
- * Records arrive through tec_bulk_push_named or tec_bam_count(b, 3, ...) only; the other pushes, tec_bam_count in modes
- * 0-2 and tec_bam_count_range return TEC_ERR_STATE until the next begin.  tec_bulk_finish and tec_bulk_allreduce end
+ * Records arrive through tec_bulk_push_named, tec_bam_count(b, 3, ...) or the byte ranges of mode 4 (below) only; the other
+ * pushes, and tec_bam_count and tec_bam_count_range in modes 0-2, return TEC_ERR_STATE until the next begin.  tec_bulk_finish and tec_bulk_allreduce end
  * the input: records still waiting for a mate count as no-mate.  stats[TEC_BS_NO_MATE] = excluded + no-mate records.
  * tec_get_info: "bulk_name_excluded" (excluded records), "bulk_name_pending_peak" (largest number of records waiting for
  * their mate after a batch), "bulk_name_ms" (device milliseconds of the pairing stage: sorts and group pass).  A batch
@@ -252,6 +252,10 @@ int tec_sc_import_packed_dev(tec_ctx* ctx, int64_t n, const void* records);
  *                             would have called back
  *   tec_sc_allgather_triples  after tec_sc_finalize: every rank holds the job's triples, ascending in
  *                             (ensg, cell); tec_sc_fetch returns them
+ *   tec_bulk_name_exchange    after tec_bam_count_range(b, 4, ...): partition, all-gather of the group sizes, grouped
+ *                             send / receive, import (see tec_bulk_name_partition_dev).  The ranks agree on success
+ *                             before any record moves (the receive buffer and the pairing stage's rows are allocated
+ *                             first): a rank that fails makes every rank return its status
  * Every rank must make the same sequence of these calls.  TEC_ERR_UNSUPPORTED: libnccl.so.2 not found. */
 #define TEC_COMM_ID_BYTES 128
 int tec_comm_unique_id(tec_ctx* ctx, void* id, int32_t capacity);
@@ -261,6 +265,7 @@ int tec_comm_info(tec_ctx* ctx, int32_t* rank, int32_t* world);
 int tec_bulk_allreduce(tec_ctx* ctx);
 int tec_sc_exchange(tec_ctx* ctx, int64_t* n_owned);
 int tec_sc_allgather_triples(tec_ctx* ctx, int64_t* n_triples);
+int tec_bulk_name_exchange(tec_ctx* ctx, int64_t* n_owned);
 
 /* sc_save_result's choice of rows (te_count.py:724-733): hit cells by count descending, ties by
  * ascending id, at most maxcells.  cells_out must hold min(maxcells, n_hit_cells) entries. */
@@ -301,7 +306,7 @@ int tec_sc_matrix_mtx(tec_ctx *ctx, int64_t n_cols, const uint32_t *cells, int64
  * (and tec_bam_set_whitelist) exactly as for tbam_*, tec_bulk_begin / tec_sc_begin, tec_bam_count (decodes
  * the whole file into the running count), tec_bulk_finish / tec_sc_finalize, tec_bam_close.
  * mode: 0 single end, 1 paired end, 2 single cell, 3 paired end by read name (tec_bulk_begin(ctx, 2, qual); whole files
- * only: tec_bam_count_range refuses it with TEC_ERR_ARG).  On TEC_ERR_UNSUPPORTED start over with libtecbam.
+ * only: tec_bam_count_range refuses it with TEC_ERR_ARG and takes mode 4 instead, below).  On TEC_ERR_UNSUPPORTED start over with libtecbam.
  * Options (tec_set_option): "bam_window_blocks" (BGZF blocks per pass, default 65536: 4.3 GB of inflated bytes
  * in HBM), "bam_lanes" (blocks decoded per warp, default 1).  Limits shared with libtecbam: reference_end comes
  * from the CIGAR field of the record (for alignments of more than 65535 operations that field is the placeholder
@@ -341,6 +346,26 @@ int tec_bam_count_range(tec_bam *b, int mode, int qual, int64_t byte_lo, int64_t
  * with b's chromosome map into rows 0 and 1 (the record layout above), with the same rules and the same status as the
  * device parse (TEC_ERR_FORMAT for a malformed record, TEC_ERR_ARG when a buffer is not one whole record). */
 int tec_bulk_keep_bank(tec_ctx *ctx, int bank);
+/* Paired end by read name over byte ranges.  A mate may lie in any range, so tec_bam_count_range(b, 4, ...) (after
+ * tec_bulk_begin(ctx, 2, qual)) pairs and counts nothing: the rows of the range's records (one per record, with name key and
+ * role) are appended in file order to a HELD set; out[] means what it means in single-end mode.  Then every rank:
+ *   tec_bulk_name_partition_dev(ctx, world, counts, &records)   counts the held excluded records (bulk_name_excluded,
+ *       stats[TEC_BS_NO_MATE]) and drops them, and packs the others as 32-byte records grouped by owner rank
+ *       key_lo % world (1..8 ranks; key_lo is a splitmix64 output), file order kept inside a group; counts[world] (host)
+ *       are the group sizes, *records the device buffer (valid until the next import, partition or begin on ctx);
+ *   the caller moves group r of every rank to rank r (an all-to-all), received groups laid out by source rank;
+ *   tec_bulk_name_import_dev(ctx, n, records)   takes the n received records (device pointer), which are then in file
+ *       order, and pairs them in one pass of the pairing stage; records left without a mate stay pending, so
+ *       tec_bulk_finish / tec_bulk_allreduce count them as no-mate.
+ * Summed over the ranks the counters and statistics equal those of one tec_bam_count(b, 3, ...) of the whole file.
+ * tec_bulk_name_exchange does the three steps over the communicator of tec_comm_init (below) and returns the number of
+ * records this rank received.
+ * State: while held rows wait for the partition, the pushes, tec_bam_count, tec_bulk_finish and tec_bulk_allreduce
+ * return TEC_ERR_STATE; tec_bulk_begin drops the held rows.  Mode 4 in a run that has records pushed into the pairing
+ * stage returns TEC_ERR_STATE.  The limit of 2^32 - 2^13 records per pairing pass applies to the records one rank holds
+ * and to those one owner receives (TEC_ERR_LIMIT). */
+int tec_bulk_name_partition_dev(tec_ctx *ctx, int world, int64_t *counts, void **records);
+int tec_bulk_name_import_dev(tec_ctx *ctx, int64_t n, const void *records);
 int tec_bam_range_record(const tec_bam *b, int which, void *buf, int64_t cap, int64_t *len);
 int tec_bam_pair_columns(tec_bam *b, const void *rec1, int64_t n1, const void *rec2, int64_t n2, int qual,
                          int32_t *start, int32_t *end, uint16_t *chrom, uint8_t *mapq, uint8_t *flag);

@@ -67,6 +67,9 @@ SIGNATURES = {
     "tec_bam_range_record": (ctypes.c_int, [_vp, ctypes.c_int, _vp, ctypes.c_int64, _c_i64p]),
     "tec_bam_pair_columns": (ctypes.c_int, [_vp, _vp, ctypes.c_int64, _vp, ctypes.c_int64, ctypes.c_int, _vp, _vp, _vp, _vp, _vp]),
     "tec_bulk_keep_bank": (ctypes.c_int, [_vp, ctypes.c_int]),
+    "tec_bulk_name_partition_dev": (ctypes.c_int, [_vp, ctypes.c_int, _c_i64p, ctypes.POINTER(_vp)]),
+    "tec_bulk_name_import_dev": (ctypes.c_int, [_vp, ctypes.c_int64, _vp]),
+    "tec_bulk_name_exchange": (ctypes.c_int, [_vp, _c_i64p]),
     "tec_bam_info": (ctypes.c_int64, [_vp, ctypes.c_int]),
     "tec_sc_matrix_text": (ctypes.c_int, [_vp, ctypes.c_int64, _c_u32p, ctypes.c_char_p, _c_i64p, _c_i64p]),
     "tec_sc_matrix_read": (ctypes.c_int, [_vp, ctypes.c_int64, ctypes.c_int64, _vp]),
@@ -190,7 +193,8 @@ class DeviceBam:
         """The records that start in the BGZF blocks of [byte_lo, byte_hi) (include/tecount.h: tec_bam_count_range).
         Returns {n, start, exit, size}: start / exit are (block file offset, offset in the inflated block).  Paired end
         (mode 1) adds first / last: the raw bytes of the range's first and last record (b"" without records); the
-        engine then waits for Engine.bulk_keep_bank."""
+        engine then waits for Engine.bulk_keep_bank.  Paired end by read name (mode 4, after bulk_begin(..., pairing='name'))
+        holds the range's rows unpaired; the engine then waits for Engine.bulk_name_partition_dev (or bulk_name_exchange)."""
         out = (ctypes.c_int64 * 6)()
         rc = self._lib.tec_bam_count_range(self._h, int(mode), int(qual), int(byte_lo), int(byte_hi), out)
         if rc != 0:
@@ -394,6 +398,17 @@ class Engine:
         """after a paired-end count_range: keep counter bank `bank` (the parity of the range's global record offset)"""
         self._check(self._lib.tec_bulk_keep_bank(self._h, int(bank)))
 
+    def bulk_name_partition_dev(self, world):
+        """after count_range(4, ...): (counts per owner rank, device pointer of the packed 32-byte records)"""
+        counts = (ctypes.c_int64 * world)()
+        p = _vp()
+        self._check(self._lib.tec_bulk_name_partition_dev(self._h, int(world), counts, ctypes.byref(p)))
+        return list(counts), (p.value or 0)
+
+    def bulk_name_import_dev(self, n, records):
+        """the n records this rank owns (device pointer, laid out by source rank), paired in one pass"""
+        self._check(self._lib.tec_bulk_name_import_dev(self._h, int(n), records))
+
     def bulk_counts_dev(self):
         return self._lib.tec_bulk_counts_dev(self._h)
 
@@ -507,6 +522,13 @@ class Engine:
     def bulk_allreduce(self):
         """sum of the ranks' counter blocks in place (behind the pushes, on the library's stream)"""
         self._check(self._lib.tec_bulk_allreduce(self._h))
+
+    def bulk_name_exchange(self):
+        """after count_range(4, ...) on every rank: the rows exchanged by name owner and paired; returns the number of
+        records this rank received"""
+        n = ctypes.c_int64(0)
+        self._check(self._lib.tec_bulk_name_exchange(self._h, ctypes.byref(n)))
+        return n.value
 
     def sc_exchange(self):
         """all-to-all of the survivors by owner rank; returns the number of records this rank now owns"""

@@ -275,7 +275,8 @@ inline int parse_pair(Reader& r, const uint8_t* rec1, int64_t n1, const uint8_t*
  *   int  parse(const BlockDesc*, int n_blocks, const BlockChain* used, const int64_t* base, int64_t n_records, int64_t w_end,
  *              int mode, int qual, const Reader&, int* err, int64_t* err_rec)                 parse_record per record into the columns
  *   int  deliver(int64_t n_records, int mode)                          hand the columns on (tec_*_push_dev / copy out; MODE_PE_NAME:
- *                                                                      the rows, keys and roles to the pairing stage, pair_name.cuh)
+ *                                                                      the rows, keys and roles to the pairing stage, pair_name.cuh;
+ *                                                                      MODE_PE_NAME_RANGE: the same rows appended to its held set)
  * and for paired-end byte ranges (decode_range with MODE_PE):
  *   int  parse_pairs(const BlockChain*, const int64_t* base, int nb, int64_t n_records, int64_t g0, int qual, const Reader&,
  *                    int* err, int64_t* err_rec)                       parse_adjacent_pair per adjacent pair into the two column sets
@@ -432,6 +433,8 @@ int decode_all(Reader& r, Backend& be, int mode, int qual, int window_blocks, in
 // column set j & 1 (parse_pairs / deliver_pairs: two counter banks); the caller keeps the set of the range's global
 // offset once it is known, and parses the pair across the border from the raw first / last records kept here.  The last
 // complete record of a window is carried into the next one, so the pair across two windows is formed exactly once.
+// Paired end by read name (MODE_PE_NAME_RANGE): a mate may lie in any range, so the range pairs nothing; its rows are
+// delivered one per record, as in single end, and the caller exchanges them by name owner before they are paired.
 constexpr int RANGE_TAIL_BLOCKS = 16;               // blocks behind the range that are inflated for its last record:
 constexpr size_t RANGE_TAIL_BYTES = size_t(1) << 20;   // at least 16 of them and at least 1 MiB of inflated data
 struct RangeResult {
@@ -465,6 +468,8 @@ int decode_range(Reader& r, Backend& be, int mode, int qual, int window_blocks, 
     if (!r.have_map) return r.fail(E_ARG, "the chromosome map has not been set");
     if (!res || lo > hi) return r.fail(E_ARG, "bad byte range");
     if (mode == bgzfdev::MODE_PE_NAME) return r.fail(E_ARG, "pairing by read name needs the whole file: no byte ranges");
+    // MODE_PE_NAME_RANGE: one MODE_PE_NAME row per record, delivered under the range mode (the rows are held, not paired)
+    const int parse_mode = mode == bgzfdev::MODE_PE_NAME_RANGE ? bgzfdev::MODE_PE_NAME : mode;
     if (window_blocks < 1) window_blocks = 1;
     *res = RangeResult();
     const bool paired = mode == bgzfdev::MODE_PE;
@@ -631,7 +636,7 @@ int decode_range(Reader& r, Backend& be, int mode, int qual, int window_blocks, 
         } else if (n_rec) {
             int err = 0;
             int64_t err_rec = -1;
-            if (be.parse(blocks.data(), nc, chain.data(), base.data(), n_rec, w_end, mode, qual, r, &err, &err_rec))
+            if (be.parse(blocks.data(), nc, chain.data(), base.data(), n_rec, w_end, parse_mode, qual, r, &err, &err_rec))
                 return r.fail(E_BACKEND, "backend: parse pass failed");
             if (err) {
                 char buf[96];

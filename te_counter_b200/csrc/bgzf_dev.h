@@ -664,7 +664,9 @@ struct ParseCtx {
     WhitelistView wl;
 };
 
-enum { MODE_SE = 0, MODE_PE = 1, MODE_SC = 2, MODE_PE_NAME = 3 };
+// MODE_PE_NAME_RANGE: byte ranges only (bam_orch.h decode_range): records are parsed as MODE_PE_NAME and the rows are
+// held for the exchange by name owner instead of being paired (pair_name.cuh)
+enum { MODE_SE = 0, MODE_PE = 1, MODE_SC = 2, MODE_PE_NAME = 3, MODE_PE_NAME_RANGE = 4 };
 
 // Record at window offset p (complete by construction) into row k.  For MODE_PE the caller passes
 // the FIRST mate and p2 = offset of the second; rows k and k + 1 are written.  MODE_PE_NAME writes the

@@ -131,6 +131,7 @@ extern "C" int tec_bulk_allreduce(tec_ctx* ctx) {
     if (!ctx) return TEC_ERR_ARG;
     if (!ctx->bulk_active) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_allreduce: tec_bulk_begin not called");
     if (ctx->bank_pending) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_allreduce: a paired-end range count waits for tec_bulk_keep_bank");
+    if (ctx->name_held) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_allreduce: rows of a read-name range wait for tec_bulk_name_partition_dev");
     if (!ctx->comm) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_allreduce: tec_comm_init not called");
     TEC_CUDA(cudaSetDevice(ctx->device));
     if (int rc = name_flush(ctx)) return rc;

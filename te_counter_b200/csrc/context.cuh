@@ -158,6 +158,7 @@ struct tec_ctx {
     bool bank_pending = false;            // a paired-end range count waits for tec_bulk_keep_bank
     bool name_pairing = false;            // tec_bulk_begin(ctx, 2, qual): mates paired by read name (pair_name.cuh)
     NameState* name = nullptr;
+    bool name_held = false;               // tec_bam_count_range mode 4 holds rows that wait for tec_bulk_name_partition_dev
     u32* d_slow_list = nullptr;           // [0] = count, then unit indices flagged for bulk_slow_kernel
     int64_t slow_cap = 0;                 // words
     void* d_ring = nullptr;               // per-warp second deferral ring of the fast bulk kernel (QEnt)

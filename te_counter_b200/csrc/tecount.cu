@@ -335,6 +335,7 @@ extern "C" int tec_bulk_begin(tec_ctx* ctx, int paired, int qual) {
     ctx->name_pairing = paired == 2;
     ctx->qual = qual;
     ctx->bulk_active = false;
+    ctx->name_held = false;
     if (ctx->name_pairing)
         if (int rc = name_begin(ctx)) return rc;
     TEC_CUDA(cudaMemsetAsync(ctx->d_counts, 0, ((size_t)ctx->idx.n_ensg + TEC_BULK_NSTATS) * 8, ctx->stream));
@@ -343,10 +344,12 @@ extern "C" int tec_bulk_begin(tec_ctx* ctx, int paired, int qual) {
     return TEC_OK;
 }
 
-// the checks of tec_bulk_push* / tec_bulk_finish / tec_bulk_allreduce: begun, and no paired-end range waiting for its bank
+// the checks of tec_bulk_push* / tec_bulk_finish / tec_bulk_allreduce: begun, no paired-end range waiting for its bank and no
+// read-name range rows waiting for their partition
 static int bulk_ready(tec_ctx* ctx, const char* what) {
     if (!ctx->bulk_active) TEC_FAIL(TEC_ERR_STATE, std::string(what) + ": tec_bulk_begin not called");
     if (ctx->bank_pending) TEC_FAIL(TEC_ERR_STATE, std::string(what) + ": a paired-end range count waits for tec_bulk_keep_bank");
+    if (ctx->name_held) TEC_FAIL(TEC_ERR_STATE, std::string(what) + ": rows of a read-name range wait for tec_bulk_name_partition_dev");
     return TEC_OK;
 }
 
@@ -753,8 +756,8 @@ extern "C" int64_t tec_get_info(tec_ctx* ctx, const char* key) {
 // ------------------------------------------------------------------------------------------------
 // BAM file -> counting path on the device (bamgpu.cuh)
 int BamGpuBackend::deliver(int64_t n, int mode) {
-    if (mode == bgzfdev::MODE_PE_NAME) {
-        const int rc = name_push_dev(ctx, n, col);
+    if (mode == bgzfdev::MODE_PE_NAME || mode == bgzfdev::MODE_PE_NAME_RANGE) {
+        const int rc = mode == bgzfdev::MODE_PE_NAME ? name_push_dev(ctx, n, col) : name_hold_dev(ctx, n, col);
         nomem = rc == TEC_ERR_NOMEM;
         return rc ? 1 : 0;
     }
@@ -856,10 +859,16 @@ extern "C" int tec_bam_count_range(tec_bam* b, int mode, int qual, int64_t byte_
     tec_ctx* ctx = b->ctx;
     if (!out) TEC_FAIL(TEC_ERR_ARG, "tec_bam_count_range: out must hold TEC_BAM_RANGE_WORDS values");
     for (int i = 0; i < TEC_BAM_RANGE_WORDS; i++) out[i] = 0;
-    if (mode < 0 || mode > 2) TEC_FAIL(TEC_ERR_ARG, "tec_bam_count_range: mode must be 0 (single end), 1 (paired end) or 2 (single cell)");
+    if (mode < 0 || mode > 4 || mode == bgzfdev::MODE_PE_NAME)
+        TEC_FAIL(TEC_ERR_ARG, "tec_bam_count_range: mode must be 0 (single end), 1 (paired end), 2 (single cell) or 4 (paired end by read "
+                              "name, rows held for the exchange)");
     if (byte_lo < 0 || byte_hi < byte_lo) TEC_FAIL(TEC_ERR_ARG, "tec_bam_count_range: bad byte range");
     if (mode == bgzfdev::MODE_SC) {
         if (!ctx->sc || !ctx->sc->active) TEC_FAIL(TEC_ERR_STATE, "tec_bam_count_range: tec_sc_begin not called");
+    } else if (mode == bgzfdev::MODE_PE_NAME_RANGE) {
+        if (!ctx->bulk_active || !ctx->name_pairing) TEC_FAIL(TEC_ERR_STATE, "tec_bam_count_range: mode 4 needs tec_bulk_begin(ctx, 2, qual)");
+        if (ctx->name->pending && !ctx->name_held)
+            TEC_FAIL(TEC_ERR_STATE, "tec_bam_count_range: mode 4 after records were pushed into this run");
     } else if (!ctx->bulk_active || (ctx->paired ? 1 : 0) != mode || ctx->name_pairing) {
         TEC_FAIL(TEC_ERR_STATE, "tec_bam_count_range: tec_bulk_begin not called for this mode");
     } else if (int st = bulk_ready(ctx, "tec_bam_count_range")) {
@@ -875,6 +884,7 @@ extern "C" int tec_bam_count_range(tec_bam* b, int mode, int qual, int64_t byte_
         TEC_CUDA(cudaMemcpyAsync(ctx->d_bank1, ctx->d_counts, bytes, cudaMemcpyDeviceToDevice, ctx->stream));
         ctx->bank_pending = true;
     }
+    if (mode == bgzfdev::MODE_PE_NAME_RANGE) ctx->name_held = true;
     bamorch::RangeResult r;
     const int rc = bamorch::decode_range(b->reader, b->be, mode, qual, ctx->opt_bam_window_blocks, (uint64_t)byte_lo, (uint64_t)byte_hi, &r);
     out[0] = r.n_records; out[1] = r.start_block; out[2] = r.start_off; out[3] = r.exit_block; out[4] = r.exit_off;

@@ -69,6 +69,26 @@ def allreduce_counts_host(counts, stats, group=None):
     return out[:len(counts)].copy(), out[len(counts):].copy()
 
 
+def bulk_name_exchange(engine, device, group=None):
+    """Paired end by read name over byte ranges (include/tecount.h tec_bulk_name_partition_dev): after every rank's
+    DeviceBam.count_range(4, ...), the rows go to the rank that owns their read name and each owner pairs what it
+    receives.  Returns the number of records this rank received.  Collective."""
+    import torch
+    import torch.distributed as dist
+    rank, world = dist.get_rank(group), dist.get_world_size(group)
+    if engine.comm_world()[1] == world and world > 1:        # comm_init was called: everything inside the library
+        return engine.bulk_name_exchange()
+    send, ptr = engine.bulk_name_partition_dev(world)
+    src = _dev_tensor(ptr, sum(send) * 4, "<i8", device)         # 4 x int64 per record
+    parts = [None] * world                                       # gloo (ranks that share a GPU): through the host
+    dist.all_gather_object(parts, [x.cpu() for x in torch.split(src, [x * 4 for x in send])], group=group)
+    dst = torch.cat([parts[r][rank] for r in range(world)]).to(device)
+    torch.cuda.synchronize(device)
+    n = int(dst.numel() // 4)
+    engine.bulk_name_import_dev(n, dst.data_ptr() if n else None)
+    return n
+
+
 # ------------------------------------------------------------------------------------ single cell
 # One process per GPU.  Each rank pushes its slice of the (coordinate-sorted) file; the survivors of
 # Part 1's filter are then exchanged by cell id (all-to-all) with their position in the job-wide

@@ -14,6 +14,10 @@ index j into bank j & 1), and once the gathered record counts give its global of
 rank in front that has records: the ranks hand out their first and last records with their range info, and the rank
 parses that pair on the host and counts it.
 
+Paired end by read name (parse_bampe(pairing='name'), mode 4): the k-th read1 of a name pairs with its k-th read2 over
+the whole file, and mates lie in any range.  So a rank's range pairs nothing: its rows are held, then sent to the rank
+that owns their name (dist.bulk_name_exchange), which pairs them in file order.  There is no pair plan.
+
 The reference has no counterpart (it is one process); results are identical to the single-GPU run, byte for byte.
 """
 import os
@@ -72,7 +76,8 @@ def count_ranges(open_and_bind, mode, qual, group=None):
     """Every rank decodes its byte range into the running count of its engine.  open_and_bind() returns the rank's
     DeviceBam (opened, chromosome map and whitelist set).  Returns (records of this rank, records of the job, pair),
     or None when a rank's decoder refused the file or the ranges do not tile it: the caller then starts over with one
-    decoder.  pair is None except in paired-end mode (1), where it is (bank to keep, columns of the border pair or None;
+    decoder.  Modes: 0 single end, 1 paired end, 2 single cell, 4 paired end by read name (rows held for the exchange).
+    pair is None except in paired-end mode (1), where it is (bank to keep, columns of the border pair or None;
     pair_plan): the caller passes the bank to Engine.bulk_keep_bank and pushes the two rows.
     Collective: every rank of the group must call it."""
     import torch.distributed as dist

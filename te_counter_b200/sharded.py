@@ -4,14 +4,15 @@ One BAM counted by all GPUs of a node:
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 --master-port 29500 \\
         -m te_counter_b200.sharded --glb genes_tes.glb --bam in.bam --mode se -o out.tsv
     ... --mode pe -o out.tsv
-    ... --mode pe --pairing name -o out.tsv      (coordinate-sorted BAM: mates paired by read name, decoded by rank 0)
+    ... --mode pe --pairing name -o out.tsv      (coordinate-sorted BAM: mates paired by read name)
     ... --mode sc --whitelist 3M-february-2018.txt --maxcells 10000 [--strand] -o out.tsv
     ... --mode sc --format mtx ... -o out_dir      (matrix.mtx.gz, features.tsv.gz, barcodes.tsv.gz; measureTE.sc_save_mtx)
 
 Every rank builds the same `measureTE` the reference's bin/te_count builds (bin/te_count:77-120) and calls the same
 method; inside, the ranks split the file by byte ranges (shard.py; paired end pairs records by their global index, so
-each rank keeps the counter bank of its record parity and counts the pair across its front border).  Rank 0 writes the outputs, which are byte for byte
-those of a one-GPU run.  With fewer GPUs than ranks the ranks share GPUs and talk over gloo (tests).
+each rank keeps the counter bank of its record parity and counts the pair across its front border; with --pairing name
+each rank sends the records of its range to the rank that owns their read name, which pairs them).  Rank 0 writes the
+outputs, which are byte for byte those of a one-GPU run.  With fewer GPUs than ranks the ranks share GPUs and talk over gloo (tests).
 """
 import argparse
 import logging
@@ -31,7 +32,8 @@ def main(argv=None):
     ap.add_argument("--format", choices=["tsv", "mtx"], default="tsv",
                     help="single cell: the reference's dense TSV (default) or a 10x-style Matrix Market directory at -o")
     ap.add_argument("--pairing", choices=["index", "name"], default="index",
-                    help="paired end: record 2i with 2i+1 as the reference (default), or mates by read name (measureTE.parse_bampe)")
+                    help="paired end: record 2i with 2i+1 as the reference (default), or mates by read name (measureTE.parse_bampe; "
+                         "every rank decodes its byte range and the records meet by name)")
     ap.add_argument("-o", "--out", required=True)
     args = ap.parse_args(argv)
     if args.format == "mtx" and args.mode != "sc":

@@ -190,26 +190,32 @@ class measureTE:
         label = 'reads' if paired else 'SE reads'
         more, done, next_log = True, 0, 1000000
         # pairing by read name: pairs are only known once the pairing stage has seen their mates, so the progress lines
-        # are written from the final pair count; a sharded run decodes the whole file on rank 0
+        # are written from the final pair count
         begin = (lambda: eng.bulk_begin(paired, qual, pairing='name')) if by_name else (lambda: eng.bulk_begin(paired, qual))
         # One file, several ranks (torch.distributed job, one process per GPU; shard.py): every rank decodes a byte range
         # on its GPU and the counters are summed; paired end keeps the counter bank of the rank's record parity and
-        # counts the pair across its front border.  Files whose ranges the decoders cannot tile are decoded by rank 0
-        # alone; the sum is the same.
+        # counts the pair across its front border; paired end by read name sends the rows of its range to the ranks that
+        # own their names, and each owner pairs what it receives.  Files whose ranges the decoders cannot tile are decoded
+        # by rank 0 alone; the sum is the same.
         rank, world = _shard.world_info()
         in_library = _shard.join_collectives(eng) if world > 1 else False
         if world > 1:
             sharded = None
-            if _device_decoder_wanted(eng) and not by_name:
+            if _device_decoder_wanted(eng):
                 def open_and_bind():
                     dev = eng.bam_open(filename)
                     dev.bind(cm)
                     return dev
-                eng.bulk_begin(paired, qual)
-                sharded = _shard.count_ranges(open_and_bind, 1 if paired else 0, qual)
+                begin()
+                sharded = _shard.count_ranges(open_and_bind, 4 if by_name else 1 if paired else 0, qual)
             if sharded is not None:
                 done, more = sharded[1], False
-                if paired:
+                if by_name:
+                    import torch
+                    from . import dist as _tdist
+                    _tdist.bulk_name_exchange(eng, torch.device('cuda', self.device))
+                    done = 0
+                elif paired:
                     bank, border = sharded[2]
                     eng.bulk_keep_bank(bank)
                     if border is not None:
@@ -288,6 +294,11 @@ class measureTE:
         log.info('{:,} Reads are QC fails'.format(int(st[_lib.BS_QCFAIL])))
         if by_name:
             excluded = eng.get_info('bulk_name_excluded')
+            if world > 1:                                     # every rank counted the excluded records it decoded
+                import torch.distributed as dist
+                parts = [None] * world
+                dist.all_gather_object(parts, excluded)
+                excluded = sum(parts)
             log.info('{:,} records were not paired by name: {:,} not primary or without exactly one mate flag, {:,} without '
                      'a mate'.format(int(st[_lib.BS_NO_MATE]), excluded, int(st[_lib.BS_NO_MATE]) - excluded))
         self.total_reads = idx

@@ -172,7 +172,8 @@ struct HostBackend {
             o_cell.insert(o_cell.end(), c_cell.begin(), c_cell.begin() + n);
             o_umi.insert(o_umi.end(), c_umi.begin(), c_umi.begin() + n);
         }
-        if (mode == bgzfdev::MODE_PE_NAME) {        // the device hands these to the pairing stage (pair_name.cuh)
+        if (mode == bgzfdev::MODE_PE_NAME || mode == bgzfdev::MODE_PE_NAME_RANGE) {     // the device hands these to the pairing
+                                                                                        // stage, or holds them (pair_name.cuh)
             o_key_hi.insert(o_key_hi.end(), c_key_hi.begin(), c_key_hi.begin() + n);
             o_key_lo.insert(o_key_lo.end(), c_key_lo.begin(), c_key_lo.begin() + n);
             o_role.insert(o_role.end(), c_role.begin(), c_role.begin() + n);
@@ -217,7 +218,8 @@ int bgzfdev_decode(void* h, int mode, int qual, int window_blocks, int64_t* n_re
     return bamorch::decode_all(s->reader, s->be, mode, qual, window_blocks, n_records);
 }
 
-// one byte range of the file (bam_orch.h decode_range); out[6] = {n_records, start_block, start_off, exit_block, exit_off, file size}
+// one byte range of the file (bam_orch.h decode_range); out[6] = {n_records, start_block, start_off, exit_block, exit_off, file size}.
+// Mode 4 (MODE_PE_NAME_RANGE): the rows, keys and roles of the range, as bgzfdev_fetch / bgzfdev_fetch_named give them
 int bgzfdev_decode_range(void* h, int mode, int qual, int window_blocks, int64_t lo, int64_t hi, int64_t* out) {
     Session* s = (Session*)h;
     bamorch::RangeResult r;
