@@ -131,8 +131,10 @@ int tec_trim(tec_ctx* ctx);
  * in, 2 = 1 + the units that two sectors answer go through a straight-line kernel first), "second_parts" (warps
  * per segment of the deferred list), "ctas_per_sm",
  * "all_hot" (counters of every ensg in shared memory when they fit), "sc_algo" (-1 auto, 0 exact search in
- * Part 3, 1 cell table), "sc_pack_umi" (2-bit UMI sort keys when possible).
- * tec_get_info: "has_stab", "stab_bytes", "has_sc_stab", "sc_stab_bytes", "n_sm", "n_features",
+ * Part 3, 1 cell table), "sc_pack_umi" (2-bit UMI sort keys when possible), "bulk_loci" (0 / 1: counts per index row,
+ * see tec_bulk_loci).
+ * tec_get_info: "has_stab", "stab_bytes", "has_sc_stab", "sc_stab_bytes", "n_sm", "n_features", "bulk_counter_words"
+ * (length of the block at tec_bulk_counts_dev),
  * "stab_primary", "stab_overflow", "stab_entries", "last_slow_units", "last_deferred_units", "last_left_units"
  * (deferred units the two-sector kernel left for the second pass), "stab_refused",
  * "sc_last_sort" (how the last tec_sc_finalize grouped the survivors by (cell, UMI): 1 one packed 64-bit key per
@@ -194,11 +196,26 @@ int tec_bulk_push(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const int32
 int tec_bulk_push_dev(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const int32_t* end,
                       const uint16_t* chrom, const uint8_t* mapq, const uint8_t* flag);
 int tec_bulk_finish(tec_ctx* ctx, int64_t* counts, int64_t* stats);
-/* device address of the int64 counters [n_ensg] followed by stats [TEC_BULK_NSTATS]; lets the
- * caller run the cross-GPU reduction (NCCL) on the library's buffer without a host round trip.
+/* device address of the int64 counters [n_ensg] followed by stats [TEC_BULK_NSTATS] (and, in a run with loci, the
+ * row counters [n_features]); lets the caller run the cross-GPU reduction (NCCL) on the library's buffer without a
+ * host round trip.  The block is tec_get_info(ctx, "bulk_counter_words") words long; a begin with loci may move it.
  * The counters are in the library's internal order (the same on every rank for the same index);
  * tec_bulk_finish returns them in ensg-id order. */
 void* tec_bulk_counts_dev(tec_ctx* ctx);
+/* Counts per index row ("loci"; an extension outside the parity claim): tec_set_option(ctx, "bulk_loci", 1) before
+ * tec_bulk_begin, read at the begin and held until the next one.  The rule, in every bulk mode (single end, paired end
+ * by index or by name):
+ *   - filters, mate merge, candidate rule, point tests, type rule and statistics are unchanged;
+ *   - a unit is counted exactly when the per-name tally adds to it: its hit rows include a gene, TE or snRNA type.
+ *     A counted unit adds 1 to every row it hits, once per row;
+ *   - a unit that is not counted adds nothing (no hit, only uncounted types, the enhancer crash unit);
+ *   - with "bulk_strand", rows the strand filter removes are not hits.
+ * So for every name e, the sum over the rows of e is at least count[e], and equal when no unit hits two rows of e;
+ * per-name counts and statistics are those of a run without loci.  The run uses the exact search kernel.  The counter
+ * block grows by n_features words (all-reduce, bank copy and name exchange carry them).
+ * tec_bulk_loci: counts[n_features] in the row order of tec_index_upload.  Same checks as tec_bulk_finish (and the same
+ * flush of rows still waiting for a mate); TEC_ERR_STATE when the run did not begin with loci. */
+int tec_bulk_loci(tec_ctx* ctx, int64_t* counts);
 /* ---- single cell (sc_parse_bamse te_count.py:298-707, sc_save_result :709-754) ------------ */
 int tec_sc_begin(tec_ctx* ctx, int qual, int strand, int64_t n_whitelist);
 int tec_sc_push(tec_ctx* ctx, int64_t n_rec, const int32_t* start, const int32_t* end,

@@ -50,6 +50,7 @@ SIGNATURES = {
     "tec_bulk_push_named": (ctypes.c_int, [_vp, ctypes.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, ctypes.c_char_p]),
     "tec_bulk_finish": (ctypes.c_int, [_vp, _c_i64p, _c_i64p]),
     "tec_bulk_counts_dev": (_vp, [_vp]),
+    "tec_bulk_loci": (ctypes.c_int, [_vp, _c_i64p]),
     "tec_sc_begin": (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int64]),
     "tec_sc_push": (ctypes.c_int, [_vp, ctypes.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "tec_sc_push_dev": (ctypes.c_int, [_vp, ctypes.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
@@ -281,6 +282,7 @@ class Engine:
         self._h = h
         self.device = device
         self.n_ensg = 0
+        self.n_features = 0
         self._pinned = []
         self._bams = []
 
@@ -360,6 +362,7 @@ class Engine:
                       ctypes.cast(_ptr(type_code, np.uint8), _c_u8p), ctypes.cast(_ptr(strand_code, np.uint8), _c_u8p),
                       int(n_ensg), int(bucket_size)))
         self.n_ensg = int(n_ensg)
+        self.n_features = int(chrom_off[int(n_chrom)])
 
     # -- bulk
     def bulk_begin(self, paired, qual, pairing="index"):
@@ -393,6 +396,13 @@ class Engine:
         self._check(self._lib.tec_bulk_finish(self._h, ctypes.cast(counts.ctypes.data, _c_i64p),
                                               ctypes.cast(stats.ctypes.data, _c_i64p)))
         return counts, stats
+
+    def bulk_loci(self):
+        """Counts per index row of a run begun with set_option('bulk_loci', 1) (include/tecount.h tec_bulk_loci):
+        int64[n_features] in the row order of the upload (GlbIndex.sorted_layout())."""
+        loci = np.zeros(self.n_features, dtype=np.int64)
+        self._check(self._lib.tec_bulk_loci(self._h, ctypes.cast(loci.ctypes.data, _c_i64p)))
+        return loci
 
     def bulk_keep_bank(self, bank):
         """after a paired-end count_range: keep counter bank `bank` (the parity of the range's global record offset)"""

@@ -75,6 +75,7 @@ __device__ __forceinline__ bool bulk_for_each_hit(const IndexView& iv, int c, in
 }
 
 #define BULK_MAX_DISTINCT 12
+#define BULK_LOCI_REG 8          // hit rows a LOCI unit keeps in registers; more are found by a second walk
 
 struct BulkStatsLocal {
     u32 units, assigned, lowq, badchrom, qcfail, crash_enh, crash_name;
@@ -82,7 +83,9 @@ struct BulkStatsLocal {
 
 // One thread per unit (record in SE, pair in PE), grid-stride.  Per-feature counters are int64 in
 // global memory (L2-resident, 8 B x n_ensg); statistics are reduced per warp, then per CTA.
-template <bool PAIRED>
+// LOCI (tec_set_option "bulk_loci", an extension outside the parity claim): a counted unit also adds 1 to every index
+// row it hits, in the u64 row counters that follow the statistics (counts + n_ensg + TEC_BULK_NSTATS, upload order).
+template <bool PAIRED, bool LOCI>
 __global__ void __launch_bounds__(256)
 bulk_count_kernel(IndexView iv, int64_t n_units, int qual, int strand_mode,
                   const int32_t* __restrict__ start, const int32_t* __restrict__ end,
@@ -93,6 +96,7 @@ bulk_count_kernel(IndexView iv, int64_t n_units, int qual, int strand_mode,
     // a feature on '+' or '-' is a candidate only for units whose first record lies on that strand (flag 0x10 = '-');
     // features with any other strand value stay candidates for both.  Restated in oracle/te_oracle_ext.py.
     BulkStatsLocal st = {0, 0, 0, 0, 0, 0, 0};
+    u64* const loci = counts + iv.n_ensg + TEC_BULK_NSTATS;
     const u32 reject = TEC_F_UNMAPPED | TEC_F_DUP | TEC_F_QCFAIL;
     for (int64_t u = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; u < n_units;
          u += (int64_t)gridDim.x * blockDim.x) {
@@ -122,6 +126,8 @@ bulk_count_kernel(IndexView iv, int64_t n_units, int qual, int strand_mode,
 
         u32 typemask = 0, nd = 0, dist[BULK_MAX_DISTINCT];
         bool overflow = false;
+        u32 nrow = 0;
+        int64_t rows[LOCI ? BULK_LOCI_REG : 1];
         bulk_for_each_hit(iv, c, loc1, loc2, [&](int64_t fi) {
             const u32 w = __ldg(iv.info + fi);
             if (other_strand(w)) return true;
@@ -132,6 +138,11 @@ bulk_count_kernel(IndexView iv, int64_t n_units, int qual, int strand_mode,
             if (!found) {
                 if (nd < BULK_MAX_DISTINCT) dist[nd++] = e; else overflow = true;
             }
+            if (LOCI) {
+#pragma unroll
+                for (int j = 0; j < BULK_LOCI_REG; ++j) if ((u32)j == nrow) rows[j] = fi;     // unrolled: stays in registers
+                ++nrow;
+            }
             return true;
         });
         if (!typemask) continue;                                                       // :128 no result
@@ -140,6 +151,18 @@ bulk_count_kernel(IndexView iv, int64_t n_units, int qual, int strand_mode,
         if (!(typemask & counted)) {
             if (typemask & (1u << TEC_T_ENHANCER)) st.crash_enh++;                     // :145-147
             continue;
+        }
+        if (LOCI) {
+            // a counted unit: +1 for every row it hits (bulk_for_each_hit lists each row once)
+            if (nrow <= BULK_LOCI_REG) {
+#pragma unroll
+                for (int j = 0; j < BULK_LOCI_REG; ++j) if ((u32)j < nrow) atomicAdd(loci + rows[j], 1ULL);
+            } else {
+                bulk_for_each_hit(iv, c, loc1, loc2, [&](int64_t fi) {
+                    if (!other_strand(__ldg(iv.info + fi))) atomicAdd(loci + fi, 1ULL);
+                    return true;
+                });
+            }
         }
         if (!overflow) {
             for (u32 i = 0; i < nd; ++i) atomicAdd(counts + dist[i], 1ULL);            // one per distinct ensg

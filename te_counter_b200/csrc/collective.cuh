@@ -125,7 +125,7 @@ static int comm_allreduce(tec_ctx* ctx, void* dev, int64_t count, int dtype, int
     return TEC_OK;
 }
 
-// Sum of every rank's bulk counter block (n_ensg counters + TEC_BULK_NSTATS statistics), in place, ordered behind the
+// Sum of every rank's bulk counter block (n_ensg counters + TEC_BULK_NSTATS statistics [+ row counters]), in place, ordered behind the
 // pushes on the library's stream: tec_bulk_finish then returns the job's result on every rank.
 extern "C" int tec_bulk_allreduce(tec_ctx* ctx) {
     if (!ctx) return TEC_ERR_ARG;
@@ -135,5 +135,5 @@ extern "C" int tec_bulk_allreduce(tec_ctx* ctx) {
     if (!ctx->comm) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_allreduce: tec_comm_init not called");
     TEC_CUDA(cudaSetDevice(ctx->device));
     if (int rc = name_flush(ctx)) return rc;
-    return comm_allreduce(ctx, ctx->d_counts, (int64_t)ctx->idx.n_ensg + TEC_BULK_NSTATS, 1, 0);
+    return comm_allreduce(ctx, ctx->d_counts, (int64_t)ctx->bulk_words(), 1, 0);
 }

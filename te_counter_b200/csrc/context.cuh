@@ -153,8 +153,10 @@ struct tec_ctx {
     // bulk
     bool bulk_active = false;
     int paired = 0, qual = 20;
-    u64* d_counts = nullptr;              // n_ensg counters (slot order) + TEC_BULK_NSTATS statistics
+    u64* d_counts = nullptr;              // the bulk counter block (bulk_words)
     u64* d_bank1 = nullptr;               // paired-end byte range: the counters of the pairs of odd range-local index (same layout)
+    int64_t counts_cap = 0, bank1_cap = 0;   // words allocated at d_counts / d_bank1
+    bool loci = false;                    // this run tallies index rows too (opt_bulk_loci at tec_bulk_begin)
     bool bank_pending = false;            // a paired-end range count waits for tec_bulk_keep_bank
     bool name_pairing = false;            // tec_bulk_begin(ctx, 2, qual): mates paired by read name (pair_name.cuh)
     NameState* name = nullptr;
@@ -177,6 +179,7 @@ struct tec_ctx {
                                           // bit 2 tally through the per-warp hit queue, bit 3 512-thread CTAs with three tiles in flight per warp,
                                           // bit 4 queue filled behind a warp prefix sum, bit 5 768-thread CTAs, bit 6 queue drained once per tile
     int opt_bulk_strand = 0;              // extension (not in the reference): strand-aware bulk counting, exact kernel only
+    int opt_bulk_loci = 0;                // extension: count per index row too (read at tec_bulk_begin), exact kernel only
     int opt_second_parts = 4;             // warps of the second bulk pass (and of bulk2_pair_kernel) per segment of the deferred list
     int opt_second_mode = 2;              // second bulk pass: register set of distinct ensg, 0 stored by position, 1 shifted in; 2: units that
                                           // two sectors answer go through the straight-line bulk2_pair_kernel first
@@ -227,6 +230,9 @@ struct tec_ctx {
         bam_stream2 = nullptr;
     }
     void free_all() { free_stage(); free_index(); free_sc(); free_name(); free_bam(); cache.trim(); }
+    // Words of the bulk counter block: n_ensg counters (slot order), TEC_BULK_NSTATS statistics and, in a run with
+    // loci, one counter per index row (upload order).  Every copy, clear and reduction of the block takes this length.
+    size_t bulk_words() const { return (size_t)idx.n_ensg + TEC_BULK_NSTATS + (loci ? (size_t)idx.n_feat : 0); }
 };
 
 inline void tec_ctx::free_stage() {
@@ -249,6 +255,8 @@ inline void tec_ctx::free_index() {
     d_counts = nullptr;
     cudaFree(d_bank1);
     d_bank1 = nullptr;
+    counts_cap = bank1_cap = 0;
+    loci = false;
     bank_pending = false;
     cudaFree(d_slow_list);
     d_slow_list = nullptr;

@@ -318,9 +318,10 @@ extern "C" int tec_index_upload(tec_ctx* ctx, int32_t n_chrom, const int64_t* ch
             }
         }
     }
-    // per-feature counters + statistics block
-    TEC_CUDA(cudaMalloc(&ctx->d_counts, ((size_t)n_ensg + TEC_BULK_NSTATS) * 8));
-    TEC_CUDA(cudaMemsetAsync(ctx->d_counts, 0, ((size_t)n_ensg + TEC_BULK_NSTATS) * 8, ctx->stream));
+    // bulk counter block; a run with loci grows it at tec_bulk_begin
+    TEC_CUDA(cudaMalloc(&ctx->d_counts, ctx->bulk_words() * 8));
+    ctx->counts_cap = (int64_t)ctx->bulk_words();
+    TEC_CUDA(cudaMemsetAsync(ctx->d_counts, 0, ctx->bulk_words() * 8, ctx->stream));
     TEC_CUDA(cudaStreamSynchronize(ctx->stream));     // host staging vectors go out of scope
     ctx->has_index = true;
     return TEC_OK;
@@ -336,9 +337,18 @@ extern "C" int tec_bulk_begin(tec_ctx* ctx, int paired, int qual) {
     ctx->qual = qual;
     ctx->bulk_active = false;
     ctx->name_held = false;
+    ctx->loci = ctx->opt_bulk_loci != 0;
     if (ctx->name_pairing)
         if (int rc = name_begin(ctx)) return rc;
-    TEC_CUDA(cudaMemsetAsync(ctx->d_counts, 0, ((size_t)ctx->idx.n_ensg + TEC_BULK_NSTATS) * 8, ctx->stream));
+    if ((int64_t)ctx->bulk_words() > ctx->counts_cap) {
+        TEC_CUDA(cudaStreamSynchronize(ctx->stream));
+        cudaFree(ctx->d_counts);
+        ctx->d_counts = nullptr;
+        ctx->counts_cap = 0;
+        TEC_CUDA(cudaMalloc(&ctx->d_counts, ctx->bulk_words() * 8));
+        ctx->counts_cap = (int64_t)ctx->bulk_words();
+    }
+    TEC_CUDA(cudaMemsetAsync(ctx->d_counts, 0, ctx->bulk_words() * 8, ctx->stream));
     ctx->bulk_active = true;
     ctx->bank_pending = false;
     return TEC_OK;
@@ -487,6 +497,17 @@ static int bulk_launch_one(tec_ctx* ctx, int64_t n_units, const int32_t* start, 
     IndexView iv = ctx->idx.view();
     u64* counts = ctx->d_counts;
     u64* stats = ctx->d_counts + ctx->idx.n_ensg;
+    if (ctx->loci) {          // the row tally lives in the exact kernel only; it also gives the per-name counts and statistics
+        const int64_t want = (n_units + 255) / 256;
+        const int blocks = (int)std::min<int64_t>(want, (int64_t)ctx->n_sm * 8);
+        if (ctx->paired)
+            bulk_count_kernel<true, true><<<blocks, 256, 0, ctx->stream>>>(iv, n_units, ctx->qual, ctx->opt_bulk_strand, start, end, chrom, mapq, flag, counts, stats);
+        else
+            bulk_count_kernel<false, true><<<blocks, 256, 0, ctx->stream>>>(iv, n_units, ctx->qual, ctx->opt_bulk_strand, start, end, chrom, mapq, flag, counts, stats);
+        ctx->launches++;
+        TEC_CUDA(cudaGetLastError());
+        return TEC_OK;
+    }
     const bool use_stab2 = !ctx->opt_bulk_strand && ctx->idx.has_stab2 && (ctx->opt_bulk_algo == -1 || ctx->opt_bulk_algo == 2) &&
                            bulk2_aligned(ctx->paired, start, end, chrom, mapq, flag);
     if (use_stab2) return bulk2_launch_one(ctx, n_units, start, end, chrom, mapq, flag);
@@ -547,9 +568,9 @@ static int bulk_launch_one(tec_ctx* ctx, int64_t n_units, const int32_t* start, 
     const int64_t want = (n_units + threads - 1) / threads;
     const int blocks = (int)std::min<int64_t>(want, (int64_t)ctx->n_sm * 8);
     if (ctx->paired)
-        bulk_count_kernel<true><<<blocks, threads, 0, ctx->stream>>>(iv, n_units, ctx->qual, ctx->opt_bulk_strand, start, end, chrom, mapq, flag, counts, stats);
+        bulk_count_kernel<true, false><<<blocks, threads, 0, ctx->stream>>>(iv, n_units, ctx->qual, ctx->opt_bulk_strand, start, end, chrom, mapq, flag, counts, stats);
     else
-        bulk_count_kernel<false><<<blocks, threads, 0, ctx->stream>>>(iv, n_units, ctx->qual, ctx->opt_bulk_strand, start, end, chrom, mapq, flag, counts, stats);
+        bulk_count_kernel<false, false><<<blocks, threads, 0, ctx->stream>>>(iv, n_units, ctx->qual, ctx->opt_bulk_strand, start, end, chrom, mapq, flag, counts, stats);
     ctx->launches++;
     TEC_CUDA(cudaGetLastError());
     return TEC_OK;
@@ -666,6 +687,19 @@ extern "C" int tec_bulk_finish(tec_ctx* ctx, int64_t* counts, int64_t* stats) {
     return TEC_OK;
 }
 
+extern "C" int tec_bulk_loci(tec_ctx* ctx, int64_t* counts) {
+    if (!ctx) return TEC_ERR_ARG;
+    if (int rc = bulk_ready(ctx, "tec_bulk_loci")) return rc;
+    if (!ctx->loci) TEC_FAIL(TEC_ERR_STATE, "tec_bulk_loci: the run did not begin with the option bulk_loci");
+    if (!counts) TEC_FAIL(TEC_ERR_ARG, "tec_bulk_loci: counts is NULL");
+    TEC_CUDA(cudaSetDevice(ctx->device));
+    if (int rc = name_flush(ctx)) return rc;
+    const size_t nf = (size_t)ctx->idx.n_feat;
+    if (nf) TEC_CUDA(cudaMemcpyAsync(counts, ctx->d_counts + ctx->idx.n_ensg + TEC_BULK_NSTATS, nf * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    TEC_CUDA(cudaStreamSynchronize(ctx->stream));
+    return TEC_OK;
+}
+
 extern "C" void* tec_bulk_counts_dev(tec_ctx* ctx) { return ctx ? (void*)ctx->d_counts : nullptr; }
 
 extern "C" int tec_bulk_keep_bank(tec_ctx* ctx, int bank) {
@@ -674,7 +708,7 @@ extern "C" int tec_bulk_keep_bank(tec_ctx* ctx, int bank) {
     if (bank != 0 && bank != 1) TEC_FAIL(TEC_ERR_ARG, "tec_bulk_keep_bank: bank must be 0 or 1");
     TEC_CUDA(cudaSetDevice(ctx->device));
     if (bank == 1)
-        TEC_CUDA(cudaMemcpyAsync(ctx->d_counts, ctx->d_bank1, ((size_t)ctx->idx.n_ensg + TEC_BULK_NSTATS) * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+        TEC_CUDA(cudaMemcpyAsync(ctx->d_counts, ctx->d_bank1, ctx->bulk_words() * 8, cudaMemcpyDeviceToDevice, ctx->stream));
     ctx->bank_pending = false;
     return TEC_OK;
 }
@@ -689,6 +723,7 @@ extern "C" int tec_set_option(tec_ctx* ctx, const char* key, int64_t value) {
     else if (k == "all_hot") { ctx->opt_all_hot = value ? 1 : 0; }
     else if (k == "sc_sort") { if (value < 0 || value > 1) TEC_FAIL(TEC_ERR_ARG, "sc_sort: 0 library sort in two stages, 1 packed keys + csrc/radix.cuh"); ctx->opt_sc_sort = (int)value; }
     else if (k == "bulk_strand") { ctx->opt_bulk_strand = value ? 1 : 0; }     // opt-in extension, outside the parity claim (bulk.cuh)
+    else if (k == "bulk_loci") { if (value < 0 || value > 1) TEC_FAIL(TEC_ERR_ARG, "bulk_loci: 0 or 1"); ctx->opt_bulk_loci = (int)value; }
     else if (k == "sc_prev_partition") { if (value < 0 || value > 2) TEC_FAIL(TEC_ERR_ARG, "sc_prev_partition: 0 random stores, 1 radix pass on large inputs, 2 always"); ctx->opt_sc_prev_partition = (int)value; }
     else if (k == "sc_sort_chunk") { if (value < 1 || value > 64) TEC_FAIL(TEC_ERR_ARG, "sc_sort_chunk: tiles per chunk of csrc/radix.cuh, 1..64"); g_rdx_chunk_tiles = (int)value; }
     else if (k == "second_parts") { if (value < 1 || value > 16) TEC_FAIL(TEC_ERR_ARG, "second_parts: 1..16"); ctx->opt_second_parts = (int)value; }
@@ -740,6 +775,7 @@ extern "C" int64_t tec_get_info(tec_ctx* ctx, const char* key) {
     if (k == "bulk_name_ms") return ctx->name_pairing && ctx->name ? (int64_t)(ctx->name->ms + 0.5) : 0;
     if (k == "sc_last_sort_passes") return ctx->sc_last_sort_passes;
     if (k == "n_features") return ctx->idx.n_feat;
+    if (k == "bulk_counter_words") return ctx->has_index ? (int64_t)ctx->bulk_words() : 0;
     if (k == "last_slow_units") {          // units the last fast-kernel launch handed to the exact kernel
         u32 n = 0;
         if (!ctx->d_slow_list) return 0;
@@ -879,8 +915,15 @@ extern "C" int tec_bam_count_range(tec_bam* b, int mode, int qual, int64_t byte_
     b->edge[1].clear();
     if (mode == bgzfdev::MODE_PE) {
         // bank 1 starts as a copy of the running count; bank 0 is the running count itself
-        const size_t bytes = ((size_t)ctx->idx.n_ensg + TEC_BULK_NSTATS) * 8;
-        if (!ctx->d_bank1) TEC_CUDA(cudaMalloc(&ctx->d_bank1, bytes));
+        const size_t bytes = ctx->bulk_words() * 8;
+        if (ctx->bank1_cap < (int64_t)ctx->bulk_words()) {
+            TEC_CUDA(cudaStreamSynchronize(ctx->stream));
+            cudaFree(ctx->d_bank1);
+            ctx->d_bank1 = nullptr;
+            ctx->bank1_cap = 0;
+            TEC_CUDA(cudaMalloc(&ctx->d_bank1, bytes));
+            ctx->bank1_cap = (int64_t)ctx->bulk_words();
+        }
         TEC_CUDA(cudaMemcpyAsync(ctx->d_bank1, ctx->d_counts, bytes, cudaMemcpyDeviceToDevice, ctx->stream));
         ctx->bank_pending = true;
     }

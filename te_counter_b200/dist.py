@@ -24,10 +24,10 @@ class _DevArray:
 
 
 def counts_tensor(engine, n_ensg, device):
-    """torch view (no copy) of the engine's device counter block: int64[n_ensg + BULK_NSTATS]."""
+    """torch view (no copy) of the engine's device counter block: int64[n_ensg + BULK_NSTATS], followed by the
+    row counters in a run with loci (its length is the library's "bulk_counter_words")."""
     import torch
-    from . import _lib
-    return torch.as_tensor(_DevArray(engine.bulk_counts_dev(), n_ensg + _lib.BULK_NSTATS, "<i8"), device=device)
+    return torch.as_tensor(_DevArray(engine.bulk_counts_dev(), engine.get_info("bulk_counter_words"), "<i8"), device=device)
 
 
 def comm_init(engine, group=None):

@@ -5,6 +5,7 @@ One BAM counted by all GPUs of a node:
         -m te_counter_b200.sharded --glb genes_tes.glb --bam in.bam --mode se -o out.tsv
     ... --mode pe -o out.tsv
     ... --mode pe --pairing name -o out.tsv      (coordinate-sorted BAM: mates paired by read name)
+    ... --mode se|pe --loci loci.tsv -o out.tsv   (also the counts per index row; measureTE.save_result_loci)
     ... --mode sc --whitelist 3M-february-2018.txt --maxcells 10000 [--strand] -o out.tsv
     ... --mode sc --format mtx ... -o out_dir      (matrix.mtx.gz, features.tsv.gz, barcodes.tsv.gz; measureTE.sc_save_mtx)
 
@@ -34,12 +35,16 @@ def main(argv=None):
     ap.add_argument("--pairing", choices=["index", "name"], default="index",
                     help="paired end: record 2i with 2i+1 as the reference (default), or mates by read name (measureTE.parse_bampe; "
                          "every rank decodes its byte range and the records meet by name)")
+    ap.add_argument("--loci", metavar="PATH",
+                    help="bulk: also count per index row and write them to PATH (measureTE.save_result_loci)")
     ap.add_argument("-o", "--out", required=True)
     args = ap.parse_args(argv)
     if args.format == "mtx" and args.mode != "sc":
         ap.error("--format mtx needs --mode sc")
     if args.pairing == "name" and args.mode != "pe":
         ap.error("--pairing name needs --mode pe")
+    if args.loci and args.mode == "sc":
+        ap.error("--loci needs --mode se or pe")
     import torch
     import torch.distributed as dist
     from . import measureTE
@@ -68,11 +73,13 @@ def main(argv=None):
     else:
         mte.load_genome()
         if args.mode == "pe":
-            res = mte.parse_bampe(args.bam, log=log, pairing=args.pairing)
+            res = mte.parse_bampe(args.bam, log=log, pairing=args.pairing, loci=bool(args.loci))
         else:
-            res = mte.parse_bamse(args.bam, log=log)
+            res = mte.parse_bamse(args.bam, log=log, loci=bool(args.loci))
         if rank == 0:
             mte.save_result_bulk(res, args.out, log=log)
+            if args.loci:
+                mte.save_result_loci(args.loci, log=log)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

@@ -26,6 +26,7 @@ import numpy as np
 from . import _lib
 from . import fastbam as _fastbam
 from . import index as _index
+from . import loci as _loci
 from . import mtx as _mtx
 from . import reads as _reads
 from . import shard as _shard
@@ -134,6 +135,7 @@ class measureTE:
         self._engine_obj = None
         self._index_on_device = False
         self.genome = None
+        self.locus_counts = None
 
     # ---------------------------------------------------------------- engine plumbing
     def _engine(self):
@@ -171,21 +173,24 @@ class measureTE:
         self.genelist_glb_filename = genelist_glb_filename
 
     # ---------------------------------------------------------------- bulk
-    def _parse_bulk(self, filename, strand, log, paired, pairing='index'):
+    def _parse_bulk(self, filename, strand, log, paired, pairing='index', loci=False):
         assert filename, 'You must specify a filename'
         if pairing not in ('index', 'name'):
             raise ValueError("pairing must be 'index' or 'name', not %r" % (pairing,))
         if strand and not self.extensions:
             raise NotImplementedError()                       # te_count.py:58-59 / :183-184
         qual = self._qual()
+        self.locus_counts = None
         eng = self._engine()
         eng.set_option('bulk_strand', 1 if strand else 0)     # extension: strand-aware candidates (exact-search kernel)
+        eng.set_option('bulk_loci', 1 if loci else 0)         # extension: counts per index row (exact-search kernel)
         try:
-            return self._parse_bulk_run(eng, filename, log, paired, qual, pairing == 'name')
+            return self._parse_bulk_run(eng, filename, log, paired, qual, pairing == 'name', loci)
         finally:
             eng.set_option('bulk_strand', 0)
+            eng.set_option('bulk_loci', 0)
 
-    def _parse_bulk_run(self, eng, filename, log, paired, qual, by_name=False):
+    def _parse_bulk_run(self, eng, filename, log, paired, qual, by_name=False, loci=False):
         cm = _reads.ChromMap(self.genome.chrom_keys)
         label = 'reads' if paired else 'SE reads'
         more, done, next_log = True, 0, 1000000
@@ -270,11 +275,13 @@ class measureTE:
         if sam is not None:
             sam.close()
         if world > 1 and in_library:
-            eng.bulk_allreduce()                              # NCCL, issued by the library on its stream
+            eng.bulk_allreduce()                              # NCCL, issued by the library on its stream (row counters too)
         counts, st = eng.bulk_finish()
+        rows = eng.bulk_loci() if loci else np.zeros(0, np.int64)
         if world > 1 and not in_library:
             from . import dist as _tdist
-            counts, st = _tdist.allreduce_counts_host(counts, st)
+            both, st = _tdist.allreduce_counts_host(np.concatenate([counts, rows]), st)
+            counts, rows = both[:len(counts)], both[len(counts):]
         if by_name:
             while int(st[_lib.BS_UNITS]) >= next_log:
                 log.info('Processed {:,} {}'.format(next_log, label))
@@ -302,20 +309,28 @@ class measureTE:
             log.info('{:,} records were not paired by name: {:,} not primary or without exactly one mate flag, {:,} without '
                      'a mate'.format(int(st[_lib.BS_NO_MATE]), excluded, int(st[_lib.BS_NO_MATE]) - excluded))
         self.total_reads = idx
+        if loci:                                              # device rows -> linearData order
+            self.locus_counts = np.empty(len(rows), np.int64)
+            self.locus_counts[self.genome.sorted_layout()['order']] = rows
         return dict(zip(self.all_feature_names, counts.tolist()))
 
-    def parse_bampe(self, filename, strand=False, log=None, pairing='index'):
+    def parse_bampe(self, filename, strand=False, log=None, pairing='index', loci=False):
         '''Load in a BAMPE file (reference te_count.py:42-165).
 
         pairing (extension): 'index' (default) pairs records as the reference does, record 2i with record 2i+1, which is
         only right for a name-collated file.  'name' pairs the k-th read1 of a read name with its k-th read2 wherever
         they lie (coordinate-sorted BAMs: STAR SortedByCoordinate, samtools sort); only primary records with exactly one
-        of the flags 0x40 / 0x80 (and 0x1) take part.  The result equals the reference's on the name-collated pairs.'''
-        return self._parse_bulk(filename, strand, log, True, pairing)
+        of the flags 0x40 / 0x80 (and 0x1) take part.  The result equals the reference's on the name-collated pairs.
+        loci (extension): also count per index row, see parse_bamse.'''
+        return self._parse_bulk(filename, strand, log, True, pairing, loci)
 
-    def parse_bamse(self, filename, strand=False, log=None):
-        '''Load in a BAMSE file (reference te_count.py:167-277)'''
-        return self._parse_bulk(filename, strand, log, False)
+    def parse_bamse(self, filename, strand=False, log=None, loci=False):
+        '''Load in a BAMSE file (reference te_count.py:167-277)
+
+        loci (extension): in the same run, count per index row (one TE copy, one gene row): every unit the per-name
+        tally counts adds 1 to each row it hits.  The returned dict is unchanged; self.locus_counts then holds
+        int64[n_features] in linearData order (None without loci) and save_result_loci writes it.'''
+        return self._parse_bulk(filename, strand, log, False, loci=loci)
 
     def save_result_bulk(self, result, out_filename, log=None):
         '''Save the data to a TSV file (reference te_count.py:279-296): name, count, CPM where
@@ -326,6 +341,20 @@ class measureTE:
             oh.write(''.join('{0}\t{1}\t{2}\n'.format(k, result[k], result[k] / per_million)
                              for k in sorted(result.keys())))
         log.info('Saved {0}'.format(out_filename))
+
+    def save_result_loci(self, out_filename, log=None):
+        '''Extension: the counts per index row of the last parse_bamse / parse_bampe(..., loci=True) as a TSV
+        (te_counter_b200/loci.py): a header, then one line per index row in linearData order -- so the files of several
+        samples on one index line up row for row -- with ensg, chromosome key, left, right, strand ('.' when the row
+        has none), count and the CPM of save_result_bulk.'''
+        assert out_filename, 'You must specify a filename'
+        if self.locus_counts is None:
+            raise ValueError('no counts per index row: call parse_bamse / parse_bampe with loci=True first')
+        text = _loci.tsv_text(self.genome, self.locus_counts, self.total_reads)
+        with open(out_filename, 'wb') as oh:
+            oh.write(text)
+        if log is not None:
+            log.info('Saved {0}'.format(out_filename))
 
     # ---------------------------------------------------------------- single cell
     def sc_parse_bamse(self,
